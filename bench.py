@@ -1,11 +1,17 @@
 #!/usr/bin/env python
 """Benchmark of the stereo-matching hot path (BASELINE.json metric: frames/s at 1920x1080, D=128, K=2).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (gray+pool, fused cost+aggregation+WTA, secondary matching,
 upscale+fill) over a batch of `--frames` synthetic random-dot frames per GPU.  Frames are sharded over
 GPUs (one process per GPU, no collective on the data path) => weak scaling.  Prints ONE JSON line.
+The timed loops run exactly K steps in all, split into `--repeats` windows.
+
+--dump-outputs DIR writes the disparity maps of the last timed step's distinct frames (the first `--distinct`) as
+DIR/disparity.npy (float32; with N GPUs, disparity_rank<r>.npy per rank): all of their rows when they fit in 48 MiB,
+else a fixed, seeded sample of whole image rows (of the [n*H, W] rows, in ascending order).  Inputs are seeded,
+so two builds can be compared output for output.
 
   value      frames/s, inputs (uint8 CHW, what a camera delivers) already resident in HBM, CUDA events
   e2e        frames/s through CudaStereoMatchingBackend.process_batch with pinned HOST tensors: every step
@@ -44,7 +50,7 @@ SMI_QUERY = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_s
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=10)
+    p.add_argument("--steps", type=int, default=50)
     p.add_argument("--warmup", type=int, default=3)
     p.add_argument("--impl", default="ours", choices=["ours", "reference"])
     p.add_argument("--frames", type=int, default=64, help="frames per step per GPU")
@@ -52,8 +58,39 @@ def parse_args():
     p.add_argument("--frames-per-launch", type=int, default=0, help="0 = library default (fills whole waves of the fused kernel)")
     p.add_argument("--distinct", type=int, default=8, help="distinct synthetic frames generated (tiled to --frames)")
     p.add_argument("--no-extras", action="store_true", help="skip cpu_baseline / reference_cuda / natural / multi-GPU legs")
-    p.add_argument("--repeats", type=int, default=5, help="the K-step timed loop is repeated this often; value = median")
-    return p.parse_args()
+    p.add_argument("--repeats", type=int, default=5,
+                   help="the K timed steps are split into this many windows; value = median window")
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's disparity maps here (.npy)")
+    args = p.parse_args()
+    if args.steps < 1 or args.repeats < 1:
+        p.error("--steps and --repeats must be positive")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+def windows(steps, repeats):
+    """Sizes of the timed windows: `steps` steps in all, over at most `repeats` windows."""
+    n = min(steps, repeats)
+    return [steps // n + (i < steps % n) for i in range(n)]
+
+
+DUMP_BYTES = 48 << 20   # per dump, over all ranks
+
+
+def dump_outputs(out, directory, rank, world):
+    """Writes the [F,H,W] float32 disparity maps `out` (a CUDA tensor) as rows of [F*H, W]: all of them, or a
+    seeded sample of whole rows (same rows in every run with the same arguments) when they exceed the budget."""
+    import numpy as np
+    import torch
+    rows = out.reshape(-1, out.shape[-1])
+    n = min(rows.shape[0], DUMP_BYTES // world // (rows.shape[1] * 4))
+    if n < rows.shape[0]:
+        pick = np.sort(np.random.default_rng(0).choice(rows.shape[0], size=n, replace=False))
+        rows = rows.index_select(0, torch.from_numpy(pick).to(rows.device))
+    os.makedirs(directory, exist_ok=True)
+    name = "disparity.npy" if world == 1 else f"disparity_rank{rank}.npy"
+    np.save(os.path.join(directory, name), rows.cpu().numpy())
 
 
 class ClockSampler:
@@ -379,43 +416,47 @@ def run_ours(args):
     in_bytes = 2 * F * 3 * H * W
     out_bytes = F * H * W * 4
 
-    # ---- device-resident throughput: REPEATS x (exactly K steps), each bracketed by barrier + synchronize; the
-    #      reported value is the median repeat (max over ranks per repeat) -------------------------------------
+    # ---- device-resident throughput: exactly K steps in REPEATS windows, each bracketed by barrier + synchronize;
+    #      the reported value is the median window (max over ranks per window) -------------------------------------
     for _ in range(max(args.warmup, 3)):
         sm.compute_disparity_batch(ld, rd, out=out_d)
     sampler = ClockSampler(local)
     barrier(world)
     if rank == 0:
         sampler.start()
+    win = windows(args.steps, args.repeats)
     rep_ms = []
-    for _ in range(args.repeats):
+    for n in win:
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier(world)
         e0.record()
-        for _ in range(args.steps):
+        for _ in range(n):
             sm.compute_disparity_batch(ld, rd, out=out_d)
         e1.record()
         barrier(world)
         rep_ms.append(max_over_ranks(e0.elapsed_time(e1), world))
     clocks = sampler.stop() if rank == 0 else None
-    ms = statistics.median(rep_ms)
-    value = world * F * args.steps / (ms * 1e-3)
-    rep_fps = sorted(world * F * args.steps / (t * 1e-3) for t in rep_ms)
+    if args.dump_outputs:
+        # frame i repeats frame i % distinct: sample the distinct ones
+        dump_outputs(out_d[:max(1, min(args.distinct, F))], args.dump_outputs, rank, world)
+    rep_fps = sorted(world * F * n / (t * 1e-3) for n, t in zip(win, rep_ms))
+    value = statistics.median(rep_fps)
+    ms_per_step = world * F / value * 1e3   # at the median window's rate
 
-    # ---- end to end from pinned host memory through the plugin API (median of 3 repeats of the K-step loop) ----------
+    # ---- end to end from pinned host memory through the plugin API (K steps in up to 3 windows, median window) -------
     for _ in range(2):
         be.process_batch(lh, rh, out=out_h)
+    e2e_win = windows(args.steps, 3)
     e2e_runs = []
-    for _ in range(3):
+    for n in e2e_win:
         barrier(world)
         t0 = time.perf_counter()
-        for _ in range(args.steps):
+        for _ in range(n):
             be.process_batch(lh, rh, out=out_h)   # synchronous: returns when out_h is complete
         torch.cuda.synchronize()
-        e2e_runs.append(max_over_ranks(time.perf_counter() - t0, world))
+        e2e_runs.append(world * F * n / max_over_ranks(time.perf_counter() - t0, world))
     barrier(world)
-    e2e_s = statistics.median(e2e_runs)
-    e2e = world * F * args.steps / e2e_s
+    e2e = statistics.median(e2e_runs)
     same = bool(torch.equal(out_h[:2], out_d[:2].cpu()))
     keep = out_h[:2].clone()
     ceiling = copy_ceiling_leg(lh, rh, out_h, max(2, args.steps // 2), world)
@@ -498,18 +539,18 @@ def run_ours(args):
         return
     line = {
         "metric": "frames/s", "value": round(value, 2), "unit": "frames/s", "n_gpus": world, "steps": args.steps,
-        "warmup": max(args.warmup, 3), "ms_per_step": round(ms / args.steps, 4), "higher_is_better": True,
+        "warmup": max(args.warmup, 3), "ms_per_step": round(ms_per_step, 4), "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": workload_config(args, wl, world),
         "impl_config": {"frames_per_launch": frames_per_launch, "fused_kernel_variant": sm.active_variant,
                         "level_screen": screened},
-        "repeats": {"n": args.repeats, "steps_each": args.steps, "value": "median", "fps_min": round(rep_fps[0], 1),
+        "repeats": {"n": len(win), "steps_each": win, "value": "median", "fps_min": round(rep_fps[0], 1),
                     "fps_median": round(value, 1), "fps_max": round(rep_fps[-1], 1),
                     "timed_seconds_total": round(sum(rep_ms) * 1e-3, 3)},
         "e2e": {"value": round(e2e, 2), "unit": "frames/s", "h2d_bytes_per_step": in_bytes,
                 "d2h_bytes_per_step": out_bytes, "api": "CudaStereoMatchingBackend.process_batch (sd_compute_host)",
-                "timer": "wall clock around the synchronous calls, max over ranks, median of 3 repeats of the K-step loop",
-                "fps_min": round(world * F * args.steps / max(e2e_runs), 1), "fps_max": round(world * F * args.steps / min(e2e_runs), 1),
+                "timer": "wall clock around the synchronous calls, max over ranks, median of up to 3 windows of the K steps",
+                "fps_min": round(min(e2e_runs), 1), "fps_max": round(max(e2e_runs), 1),
                 "matches_device_path": same,
                 "single_frame_latency_ms": round(latency_ms, 3),
                 "copy_ceiling_fps": round(ceiling, 1), "frac_of_copy_ceiling": round(e2e / ceiling, 4),

@@ -29,11 +29,16 @@ def max_abs(a, b, mask=None):
 def golden_cases():
     if not os.path.isdir(GOLDEN_DIR):
         return []
-    return sorted(f[:-4] for f in os.listdir(GOLDEN_DIR) if f.endswith(".npz"))
+    return sorted(f[:-4] for f in os.listdir(GOLDEN_DIR) if f.endswith(".npz") and not f.endswith(".volumes.npz"))
 
 
 def load_golden(name):
-    return dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz")))
+    """A case is <name>.npz, plus <name>.volumes.npz (cost, agg) where the volumes are kept apart to keep files small."""
+    g = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz")))
+    vol = os.path.join(GOLDEN_DIR, name + ".volumes.npz")
+    if os.path.exists(vol):
+        g.update(np.load(vol))
+    return g
 
 
 def oracle_config_from_array(O, arr):
