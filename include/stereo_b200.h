@@ -61,7 +61,9 @@ typedef enum sd_stage {
     SD_STAGE_WTA = 4,      /* float [Hd,Wd]  wta_disparity_selection.cu:22-30 (disparity incl. min_d/K) */
     SD_STAGE_AGG3 = 5,     /* float [Hd,Wd,3] aggregated cost at d*-1, d*, d*+1 (circular), the three
                               values secondary_matching.cu:55-58 reads from the aggregated volume */
-    SD_STAGE_REFINED = 6   /* float [Hd,Wd]  secondary_matching.cu:55-70 */
+    SD_STAGE_REFINED = 6,  /* float [Hd,Wd]  secondary_matching.cu:55-70 */
+    SD_STAGE_RIGHT = 7     /* float [H,W]    the right view's disparity map (right-image columns) of the left-right
+                              check; frame < frames_per_launch / 2; only while the check is on */
 } sd_stage;
 
 int sd_abi_version(void);
@@ -172,10 +174,25 @@ int sd_screen_stats(sd_handle *h, double *evaluated_fraction, int reset);
  * the screen is skipped for the next 32 chunks and then probed again.  Returns the chunks left in the current pause. */
 int sd_screen_paused(sd_handle *h);
 
-/* Number of kernels one sd_compute call launches for n_frames frames. */
+/* Number of kernels one sd_compute call launches for n_frames frames (with the left-right check: chunks of
+ * frames_per_launch / 2 pairs, each counted as one launch of twice its frames plus the second fill launch). */
 int sd_launches_per_call(sd_handle *h, int n_frames);
 
 int sd_frames_per_launch(sd_handle *h);
+
+/* Left-right consistency check (OpenCV's disp12MaxDiff), off by default.  With on != 0 every frame is also matched
+ * as the mirrored pair (flip(right), flip(left)) -- the same kernels and semantics -- whose output, mirrored back, is
+ * the right view's disparity map dR (right-image columns).  Each left pixel with value d = out[r][c] is then kept bit
+ * for bit if d is finite, yr = c - rint(d) (round half to even) lies in [0, W) and |d - dR[r][yr]| <= tolerance
+ * (fp32 subtraction); otherwise it is set to invalid_disparity.  This marks most occluded pixels (no partner in the
+ * right view); consistent errors such as foreground fattening at object edges remain.
+ * tolerance: full-resolution pixels, finite and >= 0 (SD_ERR_BAD_ARG otherwise); invalid_disparity: any float.
+ * Kernels A..C run once per frame and view in shared launches, so a chunk holds frames_per_launch / 2 pairs and a
+ * call costs about twice the device time; the fill writes both maps and checks in its epilogue.  Allocates the right
+ * maps of one chunk (frames_per_launch / 2 * H * W floats, readable as SD_STAGE_RIGHT); on = 0 frees them and
+ * restores the unchecked path exactly.  SD_ERR_SHAPE for a handle created with frames_per_launch = 1;
+ * SD_ERR_UNSUPPORTED together with the row-band modes (sd_set_band, sd_band_p2p_init, sd_compute_range). */
+int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_disparity);
 
 /* Level split for launches that cannot fill the GPU (one small frame, a thin row band): the unscreened specialised
  * kernel then spreads every tile's disparity levels over several blocks and a small kernel merges the partial

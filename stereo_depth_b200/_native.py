@@ -10,7 +10,7 @@ LIB_PATH = os.path.join(HERE, "csrc", "libstereo_b200.so")
 
 SD_OK, SD_ERR_BAD_ARG, SD_ERR_SHAPE, SD_ERR_CUDA, SD_ERR_NOMEM, SD_ERR_UNSUPPORTED = 0, -1, -2, -3, -4, -5
 SD_U8, SD_F32 = 0, 1
-STAGES = dict(gray_l=0, gray_r=1, pool_l=2, pool_r=3, wta=4, agg3=5, refined=6)
+STAGES = dict(gray_l=0, gray_r=1, pool_l=2, pool_r=3, wta=4, agg3=5, refined=6, right=7)
 
 CONFIG_FIELDS = ("height", "width", "downscale_factor", "min_disparity", "max_disparity",
                  "ncc_patch_radius", "sad_patch_radius", "threshold",
@@ -20,7 +20,7 @@ CONFIG_FIELDS = ("height", "width", "downscale_factor", "min_disparity", "max_di
 EXPORTS = ("sd_abi_version", "sd_config_default", "sd_dims", "sd_create", "sd_destroy", "sd_compute",
            "sd_compute_range", "sd_set_band", "sd_band_p2p_init", "sd_band_p2p_connect", "sd_band_p2p_compute", "sd_compute_host", "sd_get_stage", "sd_set_debug_volumes", "sd_set_compat", "sd_set_variant",
            "sd_launches_per_call", "sd_frames_per_launch", "sd_active_variant", "sd_set_screen", "sd_screen_active", "sd_screen_stats", "sd_screen_paused", "sd_profile_enable", "sd_profile_read", "sd_profile_read_detail", "sd_metrics", "sd_point_cloud", "sd_check_guards", "sd_stage_pointer", "sd_set_debug_screen", "sd_set_level_split", "sd_level_split",
-           "sd_last_error", "sd_last_cuda_error")
+           "sd_set_lr_check", "sd_last_error", "sd_last_cuda_error")
 
 
 class SdConfig(C.Structure):
@@ -81,6 +81,7 @@ def lib():
     L.sd_set_level_split.argtypes = [vp, ip]
     L.sd_level_split.argtypes = [vp, ip]
     L.sd_stage_pointer.argtypes = [vp, ip, ip, C.POINTER(vp)]
+    L.sd_set_lr_check.argtypes = [vp, ip, C.c_float, C.c_float]
     L.sd_check_guards.argtypes = [vp, C.POINTER(C.c_longlong)]
     L.sd_last_error.argtypes = [vp]
     L.sd_last_error.restype = C.c_char_p
@@ -198,6 +199,9 @@ class Handle:
         self.check(lib().sd_profile_read_detail(self._h, ms, n))
         names = ("gray_pool", "pad_planes", "level_screen", "cost_agg_wta", "secondary", "fill")
         return {k: (ms[i], n[i]) for i, k in enumerate(names)}
+
+    def set_lr_check(self, on, tolerance=1.0, invalid_disparity=-1.0):
+        self.check(lib().sd_set_lr_check(self._h, 1 if on else 0, tolerance, invalid_disparity))
 
     def set_level_split(self, on):
         self.check(lib().sd_set_level_split(self._h, 1 if on else 0))

@@ -77,6 +77,10 @@ struct sd_handle {
     // known pattern; sd_check_guards counts the bytes a stray store has changed (stands in for compute-sanitizer)
     bool guards;
     std::vector<std::pair<char *, size_t>> *guard_allocs;   // (raw base, payload bytes)
+    // left-right consistency check (sd_set_lr_check): a chunk holds chunk/2 frame PAIRS, each run forward and mirrored
+    bool lr;
+    float lr_tol, lr_invalid;
+    float *rmap;     // [chunk/2][H][W] right views' disparity maps of the last chunk, in mirrored orientation
     char err[640];
     int last_cuda;
 };
@@ -162,6 +166,12 @@ size_t in_bytes_per_frame(const sd_handle *h, int dtype) {
 __global__ void extract_wta(const float4 *__restrict__ w, float *__restrict__ dst, int n, float min_ds) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) dst[i] = __fadd_rn(w[i].x, min_ds);
+}
+
+// right view's map in right-image orientation from the mirrored one
+__global__ void unmirror_rows(const float *__restrict__ src, float *__restrict__ dst, int H, int W) {
+    const int c = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
+    if (c < W && r < H) dst[(size_t)r * W + c] = src[(size_t)r * W + (W - 1 - c)];
 }
 
 __global__ void extract_agg3(const float4 *__restrict__ w, const float2 *__restrict__ e, float *__restrict__ dst, int n,
@@ -295,12 +305,19 @@ int active_split(const sd_handle *h, int frames) {
     return plan_split(h, frames, true, nullptr);
 }
 
-int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int frames, float *out, cudaStream_t st,
+// Frames per launch of the left-right check: every launch runs a pair's forward and mirrored frame
+inline int lr_pairs(const sd_handle *h) { return h->chunk / 2 > 0 ? h->chunk / 2 : 1; }
+
+// With the left-right check on, `frames` counts PAIRS: kernels A..C run over 2*frames frames (forward 0..frames-1, then
+// the mirrored pairs), the fill writes the mirrored frames' maps into h->rmap and then the forward frames into `out`,
+// checked against them.
+int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int pairs, float *out, cudaStream_t st,
               int k0 = 0, int k1 = 3) {
     int rc;
     const bool full = (k0 == 0 && k1 == 3);  // per-kernel profiling only brackets complete passes
+    const int frames = h->lr ? 2 * pairs : pairs;
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
-    if (k0 <= 0 && 0 <= k1) SD_CUDA(h, launch_gray_pool(h->g, left, right, dtype, frames, h->s, st));
+    if (k0 <= 0 && 0 <= k1) SD_CUDA(h, launch_gray_pool(h->g, left, right, dtype, frames, h->s, st, h->lr ? pairs : 0));
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
     if (k0 <= 1 && 1 <= k1) {
         h->s.range_epoch = ++h->epoch;
@@ -351,7 +368,15 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
         SD_CUDA(h, launch_secondary(g2, frames, h->s, st));
     }
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
-    if (k0 <= 3 && 3 <= k1) SD_CUDA(h, launch_fill(h->g, frames, h->s, h->gv, out, st));
+    if (k0 <= 3 && 3 <= k1 && !h->lr) SD_CUDA(h, launch_fill(h->g, frames, h->s, h->gv, out, st));
+    if (k0 <= 3 && 3 <= k1 && h->lr) {
+        const size_t n = (size_t)h->g.H * h->g.W, nd = (size_t)h->g.Hd * h->g.Wd;
+        Scratch mirrored = h->s;   // the fill of frames pairs..2*pairs-1
+        mirrored.gray += (size_t)pairs * 2 * n;
+        mirrored.refined += (size_t)pairs * nd;
+        SD_CUDA(h, launch_fill(h->g, pairs, mirrored, h->gv, h->rmap, st));
+        SD_CUDA(h, launch_fill_lr(h->g, pairs, h->s, h->gv, out, LrCheck{h->rmap, h->lr_tol, h->lr_invalid}, st));
+    }
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
     return SD_OK;
 }
@@ -378,6 +403,12 @@ int host_chunk(const sd_handle *h) {
     static const int env_hc = getenv("SD_HOST_CHUNK") ? atoi(getenv("SD_HOST_CHUNK")) : 0;
     const int want = env_hc > 0 ? env_hc : 8;
     return h->chunk < want ? h->chunk : want;
+}
+
+// frames (pairs with the left-right check) per host-path chunk: the slots hold host_chunk frames, scratch 2 * pairs
+int host_chunk_frames(const sd_handle *h) {
+    const int hc = host_chunk(h);
+    return (h->lr && lr_pairs(h) < hc) ? lr_pairs(h) : hc;
 }
 
 int ensure_host_pipeline(sd_handle *h, int dtype) {
@@ -614,6 +645,7 @@ int sd_destroy(sd_handle *h) {
         scratch_free(h, h->s.bucket_count);
         scratch_free(h, h->s.screen_stats);
         scratch_free(h, h->s.range_flag);
+        scratch_free(h, h->rmap);
         if (h->prof_events) {
             for (cudaEvent_t e : *h->prof_events) cudaEventDestroy(e);
             delete h->prof_events;
@@ -636,8 +668,9 @@ int sd_compute(sd_handle *h, const void *left, const void *right, int dtype, int
     if (rc != SD_OK) return rc;
     const size_t inb = in_bytes_per_frame(h, dtype), outn = (size_t)h->g.H * h->g.W;
     // Launches of (nearly) equal size rather than full chunks plus a short remainder: behind the level screen a short
-    // launch is dominated by its heaviest tiles.
-    const int nchunks = (n_frames + h->chunk - 1) / h->chunk, base = n_frames / nchunks, extra = n_frames % nchunks;
+    // launch is dominated by its heaviest tiles.  (With the left-right check a chunk holds chunk/2 pairs.)
+    const int per = h->lr ? lr_pairs(h) : h->chunk;
+    const int nchunks = (n_frames + per - 1) / per, base = n_frames / nchunks, extra = n_frames % nchunks;
     for (int c = 0, f0 = 0; c < nchunks; c++) {
         const int nf = base + (c < extra ? 1 : 0);
         rc = run_chunk(h, (const char *)left + inb * f0, (const char *)right + inb * f0, dtype, nf, out + outn * f0, st);
@@ -655,6 +688,7 @@ int sd_compute_range(sd_handle *h, const void *left, const void *right, int dtyp
     if (last_kernel == 3 && !out) return fail(h, SD_ERR_BAD_ARG, "null output pointer");
     if (dtype != SD_U8 && dtype != SD_F32) return fail(h, SD_ERR_SHAPE, "dtype must be SD_U8 or SD_F32");
     if (n_frames <= 0 || n_frames > h->chunk) return fail(h, SD_ERR_SHAPE, "sd_compute_range handles at most frames_per_launch frames");
+    if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "sd_compute_range (row-band mode) does not support the left-right check");
     DeviceGuard dg(h->device);
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     int rc = order_after_previous(h, (cudaStream_t)stream);
@@ -674,6 +708,7 @@ int sd_set_band(sd_handle *h, int pooled_row_offset, int global_height, const fl
         memset(&h->gv, 0, sizeof(h->gv));
         return SD_OK;
     }
+    if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check (sd_set_lr_check(h, 0, ...) first)");
     if (global_height % K != 0 || h->g.H % K != 0) return fail(h, SD_ERR_UNSUPPORTED, "band mode needs heights divisible by downscale_factor");
     if (!global_left_gray) return fail(h, SD_ERR_BAD_ARG, "band mode needs the global left gray image");
     h->g.band_x_off = pooled_row_offset;
@@ -700,6 +735,7 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     if (world < 1 || world > 8 || rank < 0 || rank >= world) return fail(h, SD_ERR_BAD_ARG, "peer-memory band mode supports 1..8 ranks");
     if (dtype != SD_U8 && dtype != SD_F32) return fail(h, SD_ERR_SHAPE, "dtype must be SD_U8 or SD_F32");
     if (h->p2p.on) return fail(h, SD_ERR_BAD_ARG, "sd_band_p2p_init was already called on this handle");
+    if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check (sd_set_lr_check(h, 0, ...) first)");
     const Geom &g = h->g;
     const int esize = dtype == SD_U8 ? 1 : 4, K = g.K;
     if ((g.W * esize) % 16 != 0 || g.W % 4 != 0) return fail(h, SD_ERR_UNSUPPORTED, "peer-memory band mode needs 16-byte image rows");
@@ -846,7 +882,7 @@ int sd_compute_host(sd_handle *h, const void *left, const void *right, int dtype
     // Copies of a chunk cannot overlap its own kernels, so the host path uses chunks of at most 8 frames (the
     // device path's larger default only matters for the fused kernel's wave quantisation).
     static const int env_edge = getenv("SD_HOST_EDGE") ? atoi(getenv("SD_HOST_EDGE")) : 0;   // tuning knob
-    const int hc = host_chunk(h);
+    const int hc = host_chunk_frames(h);
     const int edge = (hc >= 4 && n_frames >= 3 * hc) ? (env_edge > 0 ? env_edge : 2) : hc;
     int it = 0;
     // On any failure below, copies to / from the caller's host buffers may still be in flight: drain before returning.
@@ -895,6 +931,8 @@ int sd_get_stage(sd_handle *h, int stage, int frame, float *dst, void *stream) {
     if (!h) return SD_ERR_BAD_ARG;
     if (!dst) return fail(h, SD_ERR_BAD_ARG, "null destination");
     if (frame < 0 || frame >= h->chunk) return fail(h, SD_ERR_SHAPE, "frame index outside the chunk");
+    if (stage == SD_STAGE_RIGHT && !h->lr) return fail(h, SD_ERR_UNSUPPORTED, "the right view's map exists only with the left-right check on");
+    if (stage == SD_STAGE_RIGHT && frame >= lr_pairs(h)) return fail(h, SD_ERR_SHAPE, "frame index outside the chunk (frames_per_launch / 2 pairs)");
     DeviceGuard dg(h->device);
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = (cudaStream_t)stream;
@@ -927,6 +965,10 @@ int sd_get_stage(sd_handle *h, int stage, int frame, float *dst, void *stream) {
         case SD_STAGE_REFINED:
             SD_CUDA(h, cudaMemcpyAsync(dst, h->s.refined + frame * nd, nd * 4, cudaMemcpyDeviceToDevice, st));
             break;
+        case SD_STAGE_RIGHT:
+            unmirror_rows<<<dim3((g.W + 255) / 256, g.H), 256, 0, st>>>(h->rmap + (size_t)frame * n, dst, g.H, g.W);
+            SD_CUDA(h, cudaGetLastError());
+            break;
         default:
             return fail(h, SD_ERR_SHAPE, "unknown stage");
     }
@@ -945,6 +987,7 @@ int sd_stage_pointer(sd_handle *h, int stage, int frame, const float **ptr) {
         case SD_STAGE_POOL_L:
         case SD_STAGE_POOL_R: *ptr = h->s.pool + ((size_t)frame * 2 + (stage - SD_STAGE_POOL_L)) * nd; break;
         case SD_STAGE_REFINED: *ptr = h->s.refined + frame * nd; break;
+        case SD_STAGE_RIGHT: return fail(h, SD_ERR_UNSUPPORTED, "the right view's map is stored mirrored (use sd_get_stage)");
         default: return fail(h, SD_ERR_UNSUPPORTED, "this stage is not stored as a plain float plane (use sd_get_stage)");
     }
     return SD_OK;
@@ -978,10 +1021,13 @@ int sd_set_variant(sd_handle *h, int variant) {
 int sd_launches_per_call(sd_handle *h, int n_frames) {
     if (!h || n_frames <= 0) return 0;
     // gray+pool, [pad planes for the TMA-staged specialised kernels], [level screen], cost+agg+WTA, secondary, fill
+    // (left-right check: chunks of chunk/2 pairs, kernels A..C over both frames of a pair, + the checked fill)
     int total = 0;
-    const int nchunks = (n_frames + h->chunk - 1) / h->chunk, base = n_frames / nchunks, extra = n_frames % nchunks;
+    const int per = h->lr ? lr_pairs(h) : h->chunk;
+    const int nchunks = (n_frames + per - 1) / per, base = n_frames / nchunks, extra = n_frames % nchunks;
     for (int c = 0; c < nchunks; c++) {   // the same split as sd_compute
-        const int nf = base + (c < extra ? 1 : 0);
+        const int nf = (base + (c < extra ? 1 : 0)) * (h->lr ? 2 : 1);
+        total += h->lr ? 1 : 0;
         const bool scr = active_variant(h, nf) == 2 && screen_active(h, nf);
         // (+2 behind the screen in reference-compat mode: absolute-index targets + gather pass)
         total += 4 + (active_variant(h, nf) >= 2 ? 1 : 0) + (scr ? 1 : 0) + (scr && h->s.agg_vol ? 2 : 0) +
@@ -991,6 +1037,34 @@ int sd_launches_per_call(sd_handle *h, int n_frames) {
 }
 
 int sd_frames_per_launch(sd_handle *h) { return h ? h->chunk : 0; }
+
+int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_disparity) {
+    if (!h) return SD_ERR_BAD_ARG;
+    if (!on) {
+        if (h->rmap) {
+            DeviceGuard dg(h->device);
+            if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
+            scratch_free(h, h->rmap);
+            h->rmap = nullptr;
+        }
+        h->lr = false;
+        return SD_OK;
+    }
+    if (!(tolerance >= 0.0f && tolerance <= 3.402823466e38f)) return fail(h, SD_ERR_BAD_ARG, "tolerance must be finite and >= 0");
+    if (h->chunk < 2)
+        return fail(h, SD_ERR_SHAPE, "the left-right check runs each frame together with its mirrored pair: create the handle "
+                                     "with frames_per_launch >= 2");
+    if (h->gv.flat || h->p2p.on) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check");
+    if (!h->rmap) {
+        DeviceGuard dg(h->device);
+        if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
+        SD_CUDA(h, scratch_alloc(h, (void **)&h->rmap, (size_t)lr_pairs(h) * h->g.H * h->g.W * sizeof(float)));
+    }
+    h->lr = true;
+    h->lr_tol = tolerance;
+    h->lr_invalid = invalid_disparity;
+    return SD_OK;
+}
 
 int sd_set_level_split(sd_handle *h, int on) {
     if (!h) return SD_ERR_BAD_ARG;

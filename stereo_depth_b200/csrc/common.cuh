@@ -121,8 +121,10 @@ struct GrayView {
 };
 
 // kernel launchers (each returns cudaGetLastError())
+// mirrored > 0 (left-right check): the last `mirrored` of the `frames` frames are the mirrored pairs (flip R, flip L) of
+// caller frames 0..mirrored-1, read from the same left / right input
 cudaError_t launch_gray_pool(const Geom &g, const void *left, const void *right, int dtype, int frames,
-                             const Scratch &s, cudaStream_t st);
+                             const Scratch &s, cudaStream_t st, int mirrored = 0);
 cudaError_t launch_pad_pooled(const Geom &g, int frames, const Scratch &s, cudaStream_t st);
 cudaError_t launch_mbm_wta_generic(const Geom &g, int frames, const Scratch &s, float *dbg_cost,
                                    float *dbg_agg, cudaStream_t st);
@@ -147,6 +149,15 @@ bool mbm_wta_ws_supported(const Geom &g);
 cudaError_t launch_mbm_wta_ws(const Geom &g, int frames, const Scratch &s, cudaStream_t st);
 cudaError_t launch_secondary(const Geom &g, int frames, const Scratch &s, cudaStream_t st);
 cudaError_t launch_fill(const Geom &g, int frames, const Scratch &s, const GrayView &gv, float *out, cudaStream_t st);
+// Left-right consistency check (api.cu sd_set_lr_check) as the epilogue of the fill: right_mirrored = [frames][H][W]
+// disparity maps of the mirrored pairs (flip R, flip L); a left pixel keeps its value d only if d is finite, its partner
+// column yr = c - rint(d) lies in [0, W) and |d - right_mirrored[r][W-1-yr]| <= tolerance, else it gets `invalid`.
+struct LrCheck {
+    const float *right_mirrored;
+    float tolerance, invalid;
+};
+cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const GrayView &gv, float *out, const LrCheck &lr,
+                           cudaStream_t st);
 // peer-memory row-band exchange (band_p2p.cu)
 cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l, void *own_r, void *prev_l, void *prev_r,
                                 void *next_l, void *next_r, int row_bytes, int band_rows, int halo, int own_rows, int prev_rows,

@@ -88,9 +88,28 @@ __device__ __forceinline__ float next_sample(const Geom &g, const float *__restr
     return p;
 }
 
-template <int KT>
+// Left-right consistency check of the left value d at (r, c) of frame `frame` (LrCheck in common.cuh).  The partner is
+// read from the MIRRORED right map at column W-1-yr: for the small disparity changes within a warp the reads stay
+// contiguous.  (c - W < rint(d) <= c  <=>  0 <= yr < W, without converting a huge d to int.)
+// Column of the partner in the mirrored right map (W-1-yr), or -1 when there is none.
+__device__ __forceinline__ int lr_partner(int W, int c, float d) {
+    if (!(fabsf(d) <= 3.402823466e38f)) return -1;   // NaN, +-inf
+    const float rd = rintf(d);
+    if (!(rd <= (float)c) || !(rd > (float)(c - W))) return -1;
+    return W - 1 - (c - (int)rd);
+}
+
+__device__ __forceinline__ float lr_checked(const Geom &g, const LrCheck &lr, int frame, int r, int c, float d) {
+    const int m = lr_partner(g.W, c, d);
+    if (m < 0) return lr.invalid;
+    const float dr = __ldg(lr.right_mirrored + ((size_t)frame * g.H + r) * g.W + m);
+    return (fabsf(__fsub_rn(d, dr)) <= lr.tolerance) ? d : lr.invalid;
+}
+
+template <int KT, bool LR>
 __global__ void __launch_bounds__(256) fill_kernel(Geom g, const float *__restrict__ gray, const GrayView glg,
-                                                   const float *__restrict__ refined, float *__restrict__ out, bool vec_ok) {
+                                                   const float *__restrict__ refined, float *__restrict__ out, bool vec_ok,
+                                                   const LrCheck lr) {
     const int c4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     const int r = blockIdx.y * blockDim.y + threadIdx.y;
     const int frame = blockIdx.z;
@@ -114,6 +133,7 @@ __global__ void __launch_bounds__(256) fill_kernel(Geom g, const float *__restri
             nk_cached = nk;
         }
         v[k] = hfill_value<KT>(g, gl, r, c, nk, p, n);
+        if (LR) v[k] = lr_checked(g, lr, frame, r, c, v[k]);
     }
     if (vec_ok && c4 + 3 < g.W) {
         *reinterpret_cast<float4 *>(o) = make_float4(v[0], v[1], v[2], v[3]);
@@ -124,8 +144,10 @@ __global__ void __launch_bounds__(256) fill_kernel(Geom g, const float *__restri
 
 // K = 2 fast path: a thread produces a 2-row x 4-column output block (rows 2x, 2x+1) from 3 + 3 refined
 // disparities; the rare colour-pick branches fall back to the generic helpers above, so semantics are identical.
+template <bool LR>
 __global__ void __launch_bounds__(256) fill_k2_kernel(Geom g, const float *__restrict__ gray, const GrayView glg,
-                                                      const float *__restrict__ refined, float *__restrict__ out) {
+                                                      const float *__restrict__ refined, float *__restrict__ out,
+                                                      const LrCheck lr) {
     const int c4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4;
     const int x = blockIdx.y * blockDim.y + threadIdx.y;
     const int frame = blockIdx.z;
@@ -146,6 +168,7 @@ __global__ void __launch_bounds__(256) fill_k2_kernel(Geom g, const float *__res
         b2 = has3 ? __ldg(da - g.Wd + 2) : 0.0f;
     }
     const float thr = g.threshold;
+    float4 res[2] = {};   // (LR: both rows first, so that the 8 partner loads of the check are in flight together)
 #pragma unroll
     for (int i = 0; i < 2; i++) {
         const int r = 2 * x + i;
@@ -163,28 +186,66 @@ __global__ void __launch_bounds__(256) fill_k2_kernel(Geom g, const float *__res
         };
         const float v0 = vf(a0, b0, c4), v1 = vf(a1, b1, c4 + 2);
         const float v2 = has3 ? vf(a2, b2, c4 + 4) : next_sample<2>(g, gl, glg, disp, r, c4 + 2, v1);
-        *reinterpret_cast<float4 *>(out + (size_t)frame * plane + (size_t)r * g.W + c4) =
-            make_float4(v0, hf(v0, v1, c4 + 1), v1, hf(v1, v2, c4 + 3));
+        res[i] = make_float4(v0, hf(v0, v1, c4 + 1), v1, hf(v1, v2, c4 + 3));
+        if (!LR) *reinterpret_cast<float4 *>(out + (size_t)frame * plane + (size_t)r * g.W + c4) = res[i];
     }
+    if (LR) {
+        const int rows = g.H - 2 * x < 2 ? g.H - 2 * x : 2;
+        float d[2][4], dr[2][4];
+        int m[2][4];
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+            d[i][0] = res[i].x, d[i][1] = res[i].y, d[i][2] = res[i].z, d[i][3] = res[i].w;
+#pragma unroll
+            for (int k = 0; k < 4; k++) m[i][k] = i < rows ? lr_partner(g.W, c4 + k, d[i][k]) : -1;
+        }
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+            const float *rrow = lr.right_mirrored + ((size_t)frame * g.H + 2 * x + i) * g.W;
+#pragma unroll
+            for (int k = 0; k < 4; k++) dr[i][k] = m[i][k] >= 0 ? __ldg(rrow + m[i][k]) : 0.0f;
+        }
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+            if (i >= rows) break;
+            float o[4];
+#pragma unroll
+            for (int k = 0; k < 4; k++)
+                o[k] = (m[i][k] >= 0 && fabsf(__fsub_rn(d[i][k], dr[i][k])) <= lr.tolerance) ? d[i][k] : lr.invalid;
+            *reinterpret_cast<float4 *>(out + (size_t)frame * plane + (size_t)(2 * x + i) * g.W + c4) =
+                make_float4(o[0], o[1], o[2], o[3]);
+        }
+    }
+}
+
+template <bool LR>
+cudaError_t fill(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
+                 cudaStream_t st) {
+    dim3 block(32, 8), grid(((g.W + 3) / 4 + 31) / 32, (g.H + 7) / 8, frames);
+    const bool vec_ok = (g.W % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15u) == 0);
+    if (g.K == 2 && vec_ok) {
+        dim3 grid2((g.W / 4 + 31) / 32, (g.Hd + 7) / 8, frames);
+        fill_k2_kernel<LR><<<grid2, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, lr);
+        return cudaGetLastError();
+    }
+    switch (g.K) {
+        case 1: fill_kernel<1, LR><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok, lr); break;
+        case 2: fill_kernel<2, LR><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok, lr); break;
+        case 4: fill_kernel<4, LR><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok, lr); break;
+        default: fill_kernel<0, LR><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok, lr); break;
+    }
+    return cudaGetLastError();
 }
 
 }  // namespace
 
 cudaError_t launch_fill(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, cudaStream_t st) {
-    dim3 block(32, 8), grid(((g.W + 3) / 4 + 31) / 32, (g.H + 7) / 8, frames);
-    const bool vec_ok = (g.W % 4 == 0) && ((reinterpret_cast<uintptr_t>(out) & 15u) == 0);
-    if (g.K == 2 && vec_ok) {
-        dim3 grid2((g.W / 4 + 31) / 32, (g.Hd + 7) / 8, frames);
-        fill_k2_kernel<<<grid2, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out);
-        return cudaGetLastError();
-    }
-    switch (g.K) {
-        case 1: fill_kernel<1><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok); break;
-        case 2: fill_kernel<2><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok); break;
-        case 4: fill_kernel<4><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok); break;
-        default: fill_kernel<0><<<grid, block, 0, st>>>(g, s.gray, gl_glob, s.refined, out, vec_ok); break;
-    }
-    return cudaGetLastError();
+    return fill<false>(g, frames, s, gl_glob, out, LrCheck{nullptr, 0.0f, 0.0f}, st);
+}
+
+cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
+                           cudaStream_t st) {
+    return fill<true>(g, frames, s, gl_glob, out, lr, st);
 }
 
 }  // namespace sd

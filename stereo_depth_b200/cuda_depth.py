@@ -10,8 +10,11 @@ Differences from the reference, all additive:
   * inputs may be uint8 as well as float32 (the reference needs the caller's `.float()`);
   * shape / dtype / device are validated (the reference silently reads out of bounds);
   * kernels run on PyTorch's current stream (the reference uses the legacy default stream);
-  * `compute_disparity_batch` processes [N,3,H,W] in one call.
+  * `compute_disparity_batch` processes [N,3,H,W] in one call;
+  * `set_left_right_check` marks occluded and mismatched pixels with an invalid value (off by default).
 """
+import math
+
 import torch
 
 from . import _native as N
@@ -64,6 +67,7 @@ class StereoMatching:
         # persistent output, like device_buffer.output_disparity (buffer/device_buffer.cc:12):
         # compute_disparity_map returns this same storage on every call
         self._out = torch.empty((self.height, self.width), dtype=torch.float32, device=self._dev())
+        self._lr_tolerance = None
 
     def _dev(self):
         return torch.device("cuda", self._device)
@@ -140,12 +144,36 @@ class StereoMatching:
         self._handle.compute_host(left_images.data_ptr(), right_images.data_ptr(), code, n, out.data_ptr())
         return out
 
+    def set_left_right_check(self, tolerance=1.0, invalid_disparity=-1.0):
+        """Left-right consistency check on every entry point of this matcher (default off).
+
+        Each frame is also matched as the mirrored pair (flip(right), flip(left)), which gives the right view's disparity
+        map; a left pixel with disparity d at column c keeps d only if d is finite, c - rint(d) is inside the image and
+        the right map there differs from d by at most `tolerance` full-resolution pixels, else it becomes
+        `invalid_disparity`.  Costs about twice the device time.  `set_left_right_check(None)` switches it off.
+        Needs a matcher created with frames_per_launch != 1 (a launch carries a frame and its mirrored pair)."""
+        if tolerance is None:
+            self._handle.set_lr_check(False)
+            self._lr_tolerance = None
+            return
+        tolerance = float(tolerance)
+        if not math.isfinite(tolerance) or tolerance < 0:
+            raise ValueError(f"tolerance must be finite and >= 0, got {tolerance}")
+        self._handle.set_lr_check(True, tolerance, float(invalid_disparity))
+        self._lr_tolerance = tolerance
+
+    @property
+    def left_right_check(self):
+        """The left-right check's tolerance in pixels, or None while the check is off."""
+        return self._lr_tolerance
+
     # ---- parity / debugging hooks (not part of the reference API) -------------------------------
     def stage(self, name, frame=0):
         H, W = self.height, self.width
         Hd, Wd, _ = self.dims
+        # ("right": the right view's disparity map of the left-right check, right-image columns)
         shape = {"gray_l": (H, W), "gray_r": (H, W), "pool_l": (Hd, Wd), "pool_r": (Hd, Wd), "wta": (Hd, Wd),
-                 "agg3": (Hd, Wd, 3), "refined": (Hd, Wd)}[name]
+                 "agg3": (Hd, Wd, 3), "refined": (Hd, Wd), "right": (H, W)}[name]
         dst = torch.empty(shape, dtype=torch.float32, device=self._dev())
         stream = torch.cuda.current_stream(self._dev()).cuda_stream
         self._handle.get_stage(name, frame, dst.data_ptr(), stream)

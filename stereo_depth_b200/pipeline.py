@@ -50,6 +50,8 @@ class DepthEstimationPipelineConfig:
     invalid_disparity: float = -1.0
     stereo_matching_backend: str = "cuda"
     log_perf_time: bool = False
+    # left-right consistency check tolerance in pixels (None = off); failing pixels get `invalid_disparity`
+    left_right_check: Optional[float] = None
 
     def update(self, **kwargs: Any) -> "DepthEstimationPipelineConfig":
         for key, value in kwargs.items():
@@ -105,7 +107,10 @@ class DepthEstimationPipeline:
                 min_disparity=self._config.min_disparity,
                 max_disparity=self._config.max_disparity,
             )
-            return CudaStereoMatchingBackend(configuration=config)
+            backend = CudaStereoMatchingBackend(configuration=config)
+            if self._config.left_right_check is not None:
+                backend.native.set_left_right_check(self._config.left_right_check, self._config.invalid_disparity)
+            return backend
         raise RuntimeError(f"Unsupported stereo matching backend: {self._config.stereo_matching_backend}")
 
 
