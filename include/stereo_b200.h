@@ -175,7 +175,8 @@ int sd_screen_stats(sd_handle *h, double *evaluated_fraction, int reset);
 int sd_screen_paused(sd_handle *h);
 
 /* Number of kernels one sd_compute call launches for n_frames frames (with the left-right check: chunks of
- * frames_per_launch / 2 pairs, each counted as one launch of twice its frames plus the second fill launch). */
+ * frames_per_launch / 2 pairs, each counted as one launch of twice its frames plus the second fill launch, plus 2 more
+ * -- the row and column passes -- with the background fill). */
 int sd_launches_per_call(sd_handle *h, int n_frames);
 
 int sd_frames_per_launch(sd_handle *h);
@@ -193,6 +194,26 @@ int sd_frames_per_launch(sd_handle *h);
  * restores the unchecked path exactly.  SD_ERR_SHAPE for a handle created with frames_per_launch = 1;
  * SD_ERR_UNSUPPORTED together with the row-band modes (sd_set_band, sd_band_p2p_init, sd_compute_range). */
 int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_disparity);
+
+/* Background fill of the pixels the left-right check rejects (KITTI devkit's interpolateBackground), off by default.
+ * A hole is a pixel the check rejects -- never a pixel whose value merely equals invalid_disparity.  In each row with a
+ * kept pixel, a run of holes gets the smaller of the two kept values that bound it (dR < dL ? dR : dL of its right and
+ * left neighbour, so the left one on ties), a run at a border its one kept neighbour; kept pixels stay bit for bit.
+ * Rows without a kept pixel above the first non-empty row copy that row, below the last one copy that row, and
+ * otherwise stay invalid_disparity (all of them in a frame without a kept pixel).  Every output value is thus a kept
+ * left value or invalid_disparity.  With on != 0 the second fill launch of a chunk writes the unchecked left maps and
+ * two more launches check and fill them in place.  Allocates frames_per_launch / 2 * H bytes of row flags, freed with
+ * the check.  SD_ERR_UNSUPPORTED while the check is off; sd_set_lr_check(h, 0, ...) also switches the fill off, and
+ * sd_set_lr_check(h, 1, ...) with the check already on keeps the fill setting. */
+int sd_set_lr_fill(sd_handle *h, int on);
+
+/* The left-right check plus the background fill (sd_set_lr_fill) without a handle: left_map = n unchecked [H][W] maps,
+ * right_map = the right views' maps in right-image columns, out = n [H][W] maps, all float32 in device memory.  out
+ * may be left_map (in place) but not right_map.  tolerance as in sd_set_lr_check.  Stream-ordered on cuda_stream
+ * (allocates n * H bytes of scratch with cudaMallocAsync).  SD_ERR_BAD_ARG for null pointers, n, H or W <= 0,
+ * n * H > INT_MAX, a tolerance that is not finite and >= 0, or out == right_map; SD_ERR_CUDA if a launch fails. */
+int sd_lr_fill(const float *left_map, const float *right_map, int n, int H, int W, float tolerance, float invalid_disparity,
+               float *out, void *cuda_stream);
 
 /* Level split for launches that cannot fill the GPU (one small frame, a thin row band): the unscreened specialised
  * kernel then spreads every tile's disparity levels over several blocks and a small kernel merges the partial

@@ -1,6 +1,9 @@
 """GPU versions of what the reference does with the disparity map after the hot path:
 accuracy metrics (depth_estimation_pipeline_metrics.py:18-56) and the point cloud
-(depth_estimation_pipeline_hooks.py:84-92, helpers/point_cloud_helpers.py:5-13)."""
+(depth_estimation_pipeline_hooks.py:84-92, helpers/point_cloud_helpers.py:5-13); and the left-right check with the
+background fill for callers that hold both views' disparity maps."""
+import math
+
 import torch
 
 from . import _native as N
@@ -42,3 +45,37 @@ def point_cloud(disparity_map: torch.Tensor, focal_length: float, baseline: floa
         _check(N.lib().sd_point_cloud(d.data_ptr(), H, W, float(baseline) * float(focal_length), float(invalid_disparity),
                                       xyz.data_ptr(), scratch.data_ptr(), stream), "sd_point_cloud")
     return xyz[: int(scratch[nb].item())]
+
+
+def left_right_fill(left_map: torch.Tensor, right_map: torch.Tensor, tolerance: float, invalid_disparity: float = -1.0,
+                    out=None):
+    """Left-right check plus background fill (StereoMatching.set_left_right_check(..., background_fill=True)) of
+    [H,W] or [N,H,W] float32 CUDA maps: `left_map` unchecked, `right_map` the right view's map in right-image columns.
+    Returns `out` (a new tensor when None); `out` may be `left_map` (in place), not `right_map`."""
+    if not (isinstance(left_map, torch.Tensor) and isinstance(right_map, torch.Tensor)):
+        raise TypeError("left_map and right_map must be tensors")
+    if (left_map.shape != right_map.shape or left_map.dim() not in (2, 3) or not left_map.is_cuda
+            or right_map.device != left_map.device):
+        raise RuntimeError("left_map and right_map must be CUDA tensors of the same [H,W] or [N,H,W] shape and device")
+    for t, name in ((left_map, "left_map"), (right_map, "right_map")):
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise RuntimeError(f"{name} must be a contiguous float32 tensor")
+    if out is None:
+        out = torch.empty_like(left_map)
+    elif (not isinstance(out, torch.Tensor) or out.shape != left_map.shape or out.dtype != torch.float32
+          or out.device != left_map.device or not out.is_contiguous()):
+        raise RuntimeError("out must be a contiguous float32 tensor of the maps' shape and device")
+    if out.data_ptr() == right_map.data_ptr():
+        raise RuntimeError("out must not be right_map")
+    tolerance = float(tolerance)
+    if not math.isfinite(tolerance) or tolerance < 0:
+        raise ValueError(f"tolerance must be finite and >= 0, got {tolerance}")
+    n = 1 if left_map.dim() == 2 else left_map.shape[0]
+    H, W = left_map.shape[-2:]
+    if n == 0 or H == 0 or W == 0:
+        return out
+    stream = torch.cuda.current_stream(left_map.device).cuda_stream
+    with torch.cuda.device(left_map.device):
+        _check(N.lib().sd_lr_fill(left_map.data_ptr(), right_map.data_ptr(), n, H, W, tolerance,
+                                  float(invalid_disparity), out.data_ptr(), stream), "sd_lr_fill")
+    return out

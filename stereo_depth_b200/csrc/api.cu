@@ -81,6 +81,8 @@ struct sd_handle {
     bool lr;
     float lr_tol, lr_invalid;
     float *rmap;     // [chunk/2][H][W] right views' disparity maps of the last chunk, in mirrored orientation
+    bool lr_fill;    // background fill of the rejected pixels (sd_set_lr_fill)
+    unsigned char *lr_rows;   // [chunk/2][H] per row: 1 if the check kept a pixel of it (the fill's column pass)
     char err[640];
     int last_cuda;
 };
@@ -310,7 +312,7 @@ inline int lr_pairs(const sd_handle *h) { return h->chunk / 2 > 0 ? h->chunk / 2
 
 // With the left-right check on, `frames` counts PAIRS: kernels A..C run over 2*frames frames (forward 0..frames-1, then
 // the mirrored pairs), the fill writes the mirrored frames' maps into h->rmap and then the forward frames into `out`,
-// checked against them.
+// checked against them (with the background fill: unchecked, then checked and filled in place by two more launches).
 int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int pairs, float *out, cudaStream_t st,
               int k0 = 0, int k1 = 3) {
     int rc;
@@ -375,7 +377,13 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
         mirrored.gray += (size_t)pairs * 2 * n;
         mirrored.refined += (size_t)pairs * nd;
         SD_CUDA(h, launch_fill(h->g, pairs, mirrored, h->gv, h->rmap, st));
-        SD_CUDA(h, launch_fill_lr(h->g, pairs, h->s, h->gv, out, LrCheck{h->rmap, h->lr_tol, h->lr_invalid}, st));
+        if (h->lr_fill) {   // unchecked left maps, then the check and the background fill in place
+            SD_CUDA(h, launch_fill(h->g, pairs, h->s, h->gv, out, st));
+            SD_CUDA(h, launch_lr_background_fill(out, h->rmap, true, pairs, h->g.H, h->g.W, h->lr_tol, h->lr_invalid, out,
+                                                 h->lr_rows, st));
+        } else {
+            SD_CUDA(h, launch_fill_lr(h->g, pairs, h->s, h->gv, out, LrCheck{h->rmap, h->lr_tol, h->lr_invalid}, st));
+        }
     }
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
     return SD_OK;
@@ -646,6 +654,7 @@ int sd_destroy(sd_handle *h) {
         scratch_free(h, h->s.screen_stats);
         scratch_free(h, h->s.range_flag);
         scratch_free(h, h->rmap);
+        scratch_free(h, h->lr_rows);
         if (h->prof_events) {
             for (cudaEvent_t e : *h->prof_events) cudaEventDestroy(e);
             delete h->prof_events;
@@ -1021,13 +1030,14 @@ int sd_set_variant(sd_handle *h, int variant) {
 int sd_launches_per_call(sd_handle *h, int n_frames) {
     if (!h || n_frames <= 0) return 0;
     // gray+pool, [pad planes for the TMA-staged specialised kernels], [level screen], cost+agg+WTA, secondary, fill
-    // (left-right check: chunks of chunk/2 pairs, kernels A..C over both frames of a pair, + the checked fill)
+    // (left-right check: chunks of chunk/2 pairs, kernels A..C over both frames of a pair, + the checked fill;
+    //  + its row and column passes with the background fill)
     int total = 0;
     const int per = h->lr ? lr_pairs(h) : h->chunk;
     const int nchunks = (n_frames + per - 1) / per, base = n_frames / nchunks, extra = n_frames % nchunks;
     for (int c = 0; c < nchunks; c++) {   // the same split as sd_compute
         const int nf = (base + (c < extra ? 1 : 0)) * (h->lr ? 2 : 1);
-        total += h->lr ? 1 : 0;
+        total += h->lr ? (h->lr_fill ? 3 : 1) : 0;
         const bool scr = active_variant(h, nf) == 2 && screen_active(h, nf);
         // (+2 behind the screen in reference-compat mode: absolute-index targets + gather pass)
         total += 4 + (active_variant(h, nf) >= 2 ? 1 : 0) + (scr ? 1 : 0) + (scr && h->s.agg_vol ? 2 : 0) +
@@ -1045,9 +1055,12 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
             DeviceGuard dg(h->device);
             if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
             scratch_free(h, h->rmap);
+            scratch_free(h, h->lr_rows);
             h->rmap = nullptr;
+            h->lr_rows = nullptr;
         }
         h->lr = false;
+        h->lr_fill = false;
         return SD_OK;
     }
     if (!(tolerance >= 0.0f && tolerance <= 3.402823466e38f)) return fail(h, SD_ERR_BAD_ARG, "tolerance must be finite and >= 0");
@@ -1063,6 +1076,33 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
     h->lr = true;
     h->lr_tol = tolerance;
     h->lr_invalid = invalid_disparity;
+    return SD_OK;
+}
+
+int sd_set_lr_fill(sd_handle *h, int on) {
+    if (!h) return SD_ERR_BAD_ARG;
+    if (!h->lr) return fail(h, SD_ERR_UNSUPPORTED, "the background fill needs the left-right check (sd_set_lr_check(h, 1, ...) first)");
+    if (on && !h->lr_rows) {
+        DeviceGuard dg(h->device);
+        if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
+        SD_CUDA(h, scratch_alloc(h, (void **)&h->lr_rows, (size_t)lr_pairs(h) * h->g.H));
+    }
+    h->lr_fill = on != 0;
+    return SD_OK;
+}
+
+int sd_lr_fill(const float *left_map, const float *right_map, int n, int H, int W, float tolerance, float invalid_disparity,
+               float *out, void *cuda_stream) {
+    if (!left_map || !right_map || !out || n <= 0 || H <= 0 || W <= 0) return SD_ERR_BAD_ARG;
+    if (!(tolerance >= 0.0f && tolerance <= 3.402823466e38f)) return SD_ERR_BAD_ARG;
+    if ((long long)n * H > 0x7fffffffLL) return SD_ERR_BAD_ARG;   // one block per row
+    if (out == right_map) return SD_ERR_BAD_ARG;                   // the row pass reads the right map while it writes
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    unsigned char *rows = nullptr;
+    if (cudaMallocAsync((void **)&rows, (size_t)n * H, st) != cudaSuccess) return SD_ERR_CUDA;
+    const cudaError_t e = launch_lr_background_fill(left_map, right_map, false, n, H, W, tolerance, invalid_disparity, out,
+                                                    rows, st);
+    if (cudaFreeAsync(rows, st) != cudaSuccess || e != cudaSuccess) return SD_ERR_CUDA;
     return SD_OK;
 }
 

@@ -158,6 +158,14 @@ struct LrCheck {
 };
 cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const GrayView &gv, float *out, const LrCheck &lr,
                            cudaStream_t st);
+// Left-right check plus background fill (DESIGN.md §13) of `frames` [H][W] maps: `left` unchecked, `right` in right-image
+// columns or, with right_mirrored, stored mirrored (partner at W-1-yr).  Each rejected pixel gets the smaller of the
+// kept values that bound its run in the row (the one neighbour at a border); rows without a kept pixel copy the nearest
+// non-empty row above the first / below the last one and otherwise stay `invalid`.  out may alias left (not right);
+// row_kept: frames*H bytes of scratch.  Two launches: the row pass and the column pass.
+cudaError_t launch_lr_background_fill(const float *left, const float *right, bool right_mirrored, int frames, int H, int W,
+                                      float tolerance, float invalid, float *out, unsigned char *row_kept,
+                                      cudaStream_t st);
 // peer-memory row-band exchange (band_p2p.cu)
 cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l, void *own_r, void *prev_l, void *prev_r,
                                 void *next_l, void *next_r, int row_bytes, int band_rows, int halo, int own_rows, int prev_rows,

@@ -218,6 +218,165 @@ __global__ void __launch_bounds__(256) fill_k2_kernel(Geom g, const float *__res
     }
 }
 
+// ---- background fill of the pixels the left-right check rejects (DESIGN.md §13) ------------------------------------
+// Row pass: one block per row, tiles of kBgTile columns, kBgItems consecutive columns per thread.  A hole's left bound
+// is the last kept column before it (block-wide exclusive max scan + the carry of earlier tiles), its right bound the
+// first kept column after it (exclusive min scan from the right).  Holes whose right bound lies beyond the tile -- the
+// row's trailing run so far -- stay pending and are written as one constant run once the bound is known (or with the
+// left bound / `invalid` after the last tile).  Holes are only written after every read of their tile, and bounds are
+// kept pixels, which the fill never changes: so `out` may alias `left`.
+constexpr int kBgThreads = 256, kBgItems = 8, kBgTile = kBgThreads * kBgItems, kBgWarps = kBgThreads / 32;
+constexpr int kNone = 0x7fffffff;
+
+// fill value of a hole bounded by the kept values da (left) and db (right): the smaller, the left one on ties
+__device__ __forceinline__ float bg_min(float da, float db) { return db < da ? db : da; }
+
+template <bool MIRRORED>
+__global__ void __launch_bounds__(kBgThreads) lr_fill_rows_kernel(const float *left, const float *__restrict__ right,
+                                                                  float *out, unsigned char *__restrict__ row_kept, int W,
+                                                                  float tolerance, float invalid) {
+    __shared__ int warp_last[kBgWarps], warp_first[kBgWarps];
+    const size_t row = blockIdx.x;
+    const float *dl = left + row * W;
+    const float *dr = right + row * W;
+    float *o = out + row * W;
+    const bool copy_kept = out != left;
+    const bool vec = W % 4 == 0 && (reinterpret_cast<uintptr_t>(left) & 15u) == 0;   // float4 loads of the row
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int carry = -1;    // last kept column of the tiles before this one
+    int pend = -1;     // first column of the pending trailing hole run
+    for (int t0 = 0; t0 < W; t0 += kBgTile) {
+        const int c0 = t0 + threadIdx.x * kBgItems;
+        float d[kBgItems];
+        if (vec && c0 + kBgItems <= W) {
+#pragma unroll
+            for (int k = 0; k < kBgItems; k += 4) {
+                const float4 v = *reinterpret_cast<const float4 *>(dl + c0 + k);
+                d[k] = v.x, d[k + 1] = v.y, d[k + 2] = v.z, d[k + 3] = v.w;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < kBgItems; k++) d[k] = c0 + k < W ? dl[c0 + k] : 0.0f;
+        }
+        int m[kBgItems];
+        float pr[kBgItems];   // (all partner loads first, so that they are in flight together)
+#pragma unroll
+        for (int k = 0; k < kBgItems; k++) m[k] = c0 + k < W ? lr_partner(W, c0 + k, d[k]) : -1;
+#pragma unroll
+        for (int k = 0; k < kBgItems; k++) pr[k] = m[k] >= 0 ? __ldg(dr + (MIRRORED ? m[k] : W - 1 - m[k])) : 0.0f;
+        unsigned keep = 0;
+        int last = -1, first = kNone;
+#pragma unroll
+        for (int k = 0; k < kBgItems; k++) {
+            const int c = c0 + k;
+            if (m[k] >= 0 && fabsf(__fsub_rn(d[k], pr[k])) <= tolerance) {
+                keep |= 1u << k;
+                last = c;
+                first = first == kNone ? c : first;
+            }
+        }
+        // exclusive scans over the threads: last kept column to the left, first kept column to the right
+        int incl_last = last, incl_first = first;
+#pragma unroll
+        for (int s = 1; s < 32; s <<= 1) {
+            const int a = __shfl_up_sync(0xffffffffu, incl_last, s);
+            const int b = __shfl_down_sync(0xffffffffu, incl_first, s);
+            if (lane >= s) incl_last = max(incl_last, a);
+            if (lane + s < 32) incl_first = min(incl_first, b);
+        }
+        int before = __shfl_up_sync(0xffffffffu, incl_last, 1);
+        int after = __shfl_down_sync(0xffffffffu, incl_first, 1);
+        if (lane == 0) before = -1;
+        if (lane == 31) after = kNone;
+        if (lane == 31) warp_last[warp] = incl_last;
+        if (lane == 0) warp_first[warp] = incl_first;
+        __syncthreads();
+        int tile_last = -1, tile_first = kNone;
+#pragma unroll
+        for (int w = 0; w < kBgWarps; w++) {
+            if (w < warp) before = max(before, warp_last[w]);
+            if (w > warp) after = min(after, warp_first[w]);
+            tile_last = max(tile_last, warp_last[w]);
+            tile_first = min(tile_first, warp_first[w]);
+        }
+        before = max(before, carry);
+        if (pend >= 0 && tile_first != kNone) {   // the pending run ends at this tile's first kept column
+            const float db = dl[tile_first];
+            const float v = carry >= 0 ? bg_min(dl[carry], db) : db;
+            for (int c = pend + threadIdx.x; c < t0; c += kBgThreads) o[c] = v;
+            pend = -1;
+        }
+        int next[kBgItems];
+        int b = after;
+#pragma unroll
+        for (int k = kBgItems - 1; k >= 0; k--) {
+            next[k] = b;
+            if (keep >> k & 1u) b = c0 + k;
+        }
+        int a = before;
+#pragma unroll
+        for (int k = 0; k < kBgItems; k++) {
+            const int c = c0 + k;
+            if (c >= W) break;
+            if (keep >> k & 1u) {
+                a = c;
+                if (copy_kept) o[c] = d[k];
+            } else if (next[k] != kNone) {
+                const float db = dl[next[k]];
+                o[c] = a >= 0 ? bg_min(dl[a], db) : db;
+            }   // else: part of the pending trailing run
+        }
+        if (tile_first == kNone) {
+            if (pend < 0) pend = t0;
+        } else {
+            carry = tile_last;
+            pend = tile_last + 1 < W ? tile_last + 1 : -1;
+        }
+        __syncthreads();   // warp_last / warp_first are rewritten by the next tile
+    }
+    if (pend >= 0) {   // a run that touches the right border: its one kept neighbour, or `invalid` in an empty row
+        const float v = carry >= 0 ? dl[carry] : invalid;
+        for (int c = pend + threadIdx.x; c < W; c += kBgThreads) o[c] = v;
+    }
+    if (threadIdx.x == 0) row_kept[row] = carry >= 0 ? 1 : 0;
+}
+
+// Column pass: a row without kept pixels copies the first non-empty row of its frame when it lies above it, the last
+// one when it lies below it; rows between non-empty rows stay `invalid`.  Blocks of non-empty rows return at once.
+__global__ void __launch_bounds__(256) lr_fill_cols_kernel(float *out, const unsigned char *__restrict__ row_kept, int H,
+                                                           int W) {
+    __shared__ int sh_first[8], sh_last[8];
+    const size_t row = blockIdx.x;
+    if (row_kept[row]) return;
+    const size_t frame = row / H;
+    const int r = (int)(row - frame * H);
+    const unsigned char *fk = row_kept + frame * H;
+    int first = kNone, last = -1;
+    for (int i = threadIdx.x; i < H; i += 256)
+        if (fk[i]) {
+            first = min(first, i);
+            last = max(last, i);
+        }
+    first = __reduce_min_sync(0xffffffffu, first);
+    last = __reduce_max_sync(0xffffffffu, last);
+    if ((threadIdx.x & 31) == 0) {
+        sh_first[threadIdx.x >> 5] = first;
+        sh_last[threadIdx.x >> 5] = last;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int w = 0; w < 8; w++) {
+        first = min(first, sh_first[w]);
+        last = max(last, sh_last[w]);
+    }
+    if (last < 0) return;   // no kept pixel in the frame: all `invalid`
+    const int src = r < first ? first : (r > last ? last : -1);
+    if (src < 0) return;
+    const float *s = out + (frame * H + src) * W;
+    float *o = out + row * W;
+    for (int c = threadIdx.x; c < W; c += 256) o[c] = s[c];
+}
+
 template <bool LR>
 cudaError_t fill(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
                  cudaStream_t st) {
@@ -246,6 +405,18 @@ cudaError_t launch_fill(const Geom &g, int frames, const Scratch &s, const GrayV
 cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
                            cudaStream_t st) {
     return fill<true>(g, frames, s, gl_glob, out, lr, st);
+}
+
+cudaError_t launch_lr_background_fill(const float *left, const float *right, bool right_mirrored, int frames, int H, int W,
+                                      float tolerance, float invalid, float *out, unsigned char *row_kept,
+                                      cudaStream_t st) {
+    const unsigned rows = (unsigned)frames * (unsigned)H;
+    if (right_mirrored)
+        lr_fill_rows_kernel<true><<<rows, kBgThreads, 0, st>>>(left, right, out, row_kept, W, tolerance, invalid);
+    else
+        lr_fill_rows_kernel<false><<<rows, kBgThreads, 0, st>>>(left, right, out, row_kept, W, tolerance, invalid);
+    lr_fill_cols_kernel<<<rows, 256, 0, st>>>(out, row_kept, H, W);
+    return cudaGetLastError();
 }
 
 }  // namespace sd

@@ -11,7 +11,8 @@ Differences from the reference, all additive:
   * shape / dtype / device are validated (the reference silently reads out of bounds);
   * kernels run on PyTorch's current stream (the reference uses the legacy default stream);
   * `compute_disparity_batch` processes [N,3,H,W] in one call;
-  * `set_left_right_check` marks occluded and mismatched pixels with an invalid value (off by default).
+  * `set_left_right_check` marks occluded and mismatched pixels with an invalid value, or fills them from the
+    background (off by default).
 """
 import math
 
@@ -68,6 +69,7 @@ class StereoMatching:
         # compute_disparity_map returns this same storage on every call
         self._out = torch.empty((self.height, self.width), dtype=torch.float32, device=self._dev())
         self._lr_tolerance = None
+        self._lr_fill = False
 
     def _dev(self):
         return torch.device("cuda", self._device)
@@ -144,28 +146,41 @@ class StereoMatching:
         self._handle.compute_host(left_images.data_ptr(), right_images.data_ptr(), code, n, out.data_ptr())
         return out
 
-    def set_left_right_check(self, tolerance=1.0, invalid_disparity=-1.0):
+    def set_left_right_check(self, tolerance=1.0, invalid_disparity=-1.0, background_fill=False):
         """Left-right consistency check on every entry point of this matcher (default off).
 
         Each frame is also matched as the mirrored pair (flip(right), flip(left)), which gives the right view's disparity
         map; a left pixel with disparity d at column c keeps d only if d is finite, c - rint(d) is inside the image and
         the right map there differs from d by at most `tolerance` full-resolution pixels, else it becomes
         `invalid_disparity`.  Costs about twice the device time.  `set_left_right_check(None)` switches it off.
-        Needs a matcher created with frames_per_launch != 1 (a launch carries a frame and its mirrored pair)."""
+        Needs a matcher created with frames_per_launch != 1 (a launch carries a frame and its mirrored pair).
+
+        background_fill=True instead gives each run of rejected pixels in a row the smaller of the two kept values that
+        bound it (occluded pixels lie on the background), a run at the image border its one kept neighbour; rows with
+        no kept pixel copy the nearest non-empty row above the first / below the last one (DESIGN.md §13).  Only rows
+        between non-empty rows, and frames without any kept pixel, keep `invalid_disparity`."""
         if tolerance is None:
             self._handle.set_lr_check(False)
             self._lr_tolerance = None
+            self._lr_fill = False
             return
         tolerance = float(tolerance)
         if not math.isfinite(tolerance) or tolerance < 0:
             raise ValueError(f"tolerance must be finite and >= 0, got {tolerance}")
         self._handle.set_lr_check(True, tolerance, float(invalid_disparity))
         self._lr_tolerance = tolerance
+        self._handle.set_lr_fill(bool(background_fill))
+        self._lr_fill = bool(background_fill)
 
     @property
     def left_right_check(self):
         """The left-right check's tolerance in pixels, or None while the check is off."""
         return self._lr_tolerance
+
+    @property
+    def background_fill(self):
+        """True while the left-right check fills the pixels it rejects instead of marking them invalid."""
+        return self._lr_fill
 
     # ---- parity / debugging hooks (not part of the reference API) -------------------------------
     def stage(self, name, frame=0):

@@ -52,6 +52,8 @@ class DepthEstimationPipelineConfig:
     log_perf_time: bool = False
     # left-right consistency check tolerance in pixels (None = off); failing pixels get `invalid_disparity`
     left_right_check: Optional[float] = None
+    # with left_right_check: fill the pixels it rejects from the background (DESIGN.md §13) instead of marking them
+    left_right_background_fill: bool = False
 
     def update(self, **kwargs: Any) -> "DepthEstimationPipelineConfig":
         for key, value in kwargs.items():
@@ -100,6 +102,9 @@ class DepthEstimationPipeline:
         return self._config
 
     def _get_stereo_matching(self) -> StereoMatching:
+        if self._config.left_right_background_fill and self._config.left_right_check is None:
+            raise RuntimeError("left_right_background_fill needs left_right_check (a tolerance in pixels): the fill "
+                               "replaces the pixels the check rejects")
         if self._config.stereo_matching_backend == "cuda":
             config = cuda_depth.StereoMatchingConfiguration(
                 height=self._config.image_shape[0],
@@ -109,7 +114,8 @@ class DepthEstimationPipeline:
             )
             backend = CudaStereoMatchingBackend(configuration=config)
             if self._config.left_right_check is not None:
-                backend.native.set_left_right_check(self._config.left_right_check, self._config.invalid_disparity)
+                backend.native.set_left_right_check(self._config.left_right_check, self._config.invalid_disparity,
+                                                    self._config.left_right_background_fill)
             return backend
         raise RuntimeError(f"Unsupported stereo matching backend: {self._config.stereo_matching_backend}")
 

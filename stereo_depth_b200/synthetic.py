@@ -42,6 +42,39 @@ def make_pair(H, W, D, seed=1234, frame=0):
     return left, right, g
 
 
+def make_layered_pair(H, W, D, seed=1234):
+    """A physically consistent scene for occlusion studies: fronto-parallel rectangles defined in the LEFT view over a
+    background at the smallest disparity, a larger disparity being nearer and drawn on top.  The right view is the
+    left one forward-warped (left column c -> right column c - d) with a z-buffer: where several left pixels land on
+    one right pixel the nearest wins.  Right pixels no left pixel reaches get fresh noise, and every right pixel gets
+    +-2 of noise.  Returns (left u8 [3,H,W], right u8 [3,H,W], gt_left float32 [H,W], visible bool [H,W]); visible is
+    False for left pixels that are occluded in the right view or land outside it."""
+    rng = np.random.default_rng(seed)
+    left = rng.integers(0, 256, (3, H, W), dtype=np.uint8)
+    lo, hi = max(1, D // 16), max(2, (3 * D) // 4)
+    gt = np.full((H, W), lo, np.int64)
+    layers = []
+    for _ in range(8):
+        h = int(rng.integers(max(2, H // 8), max(3, H // 2)))
+        w = int(rng.integers(max(2, W // 10), max(3, W // 3)))
+        r0 = int(rng.integers(0, max(1, H - h)))
+        c0 = int(rng.integers(0, max(1, W - w)))
+        layers.append((int(rng.integers(lo + 1, hi + 1)), r0, h, c0, w))
+    for d, r0, h, c0, w in sorted(layers):   # far to near
+        gt[r0:r0 + h, c0:c0 + w] = d
+    rows = np.broadcast_to(np.arange(H)[:, None], (H, W))
+    target = np.arange(W)[None, :] - gt
+    inside = target >= 0
+    zbuf = np.full((H, W), -1, np.int64)
+    np.maximum.at(zbuf, (rows[inside], target[inside]), gt[inside])
+    visible = inside & (zbuf[rows, np.where(inside, target, 0)] == gt)
+    right = rng.integers(0, 256, (3, H, W), dtype=np.uint8)
+    right[:, rows[visible], target[visible]] = left[:, rows[visible], np.nonzero(visible)[1]]
+    noise = rng.integers(-2, 3, (3, H, W), dtype=np.int16)
+    right = np.clip(right.astype(np.int16) + noise, 0, 255).astype(np.uint8)
+    return left, right, gt.astype(np.float32), visible
+
+
 def make_batch(n, H, W, D, seed=1234, first_frame=0):
     ls, rs = [], []
     for f in range(n):

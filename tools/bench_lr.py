@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Cost of the left-right consistency check (StereoMatching.set_left_right_check): check off vs on, alternated in the same
-process on the same handle.  Inputs resident in HBM, CUDA events, warm-up, median of 5 repeats.
+"""Cost of the left-right consistency check (StereoMatching.set_left_right_check): check off, on, and on with the
+background fill, alternated in the same process on the same handle.  Inputs resident in HBM, CUDA events, warm-up,
+median of 5 repeats.
 
-    python tools/bench_lr.py [--out profiles/lr_check_b200.json]
+    python tools/bench_lr.py [--out profiles/lr_fill_b200.json]
 
 Legs: C3 (1080p, D=128, 64 frames per step), C5 (720p) and C1 (480p) batches; one frame per call at 1080p and 720p; the
 per-kernel split (profile_read_detail) at C3; the host path end to end at C3; the natural pair when data/_ref has it.
@@ -54,8 +55,11 @@ def inputs(H, W, D, n, distinct=8):
     return (torch.from_numpy(np.concatenate([l] * reps)[:n]).cuda(), torch.from_numpy(np.concatenate([r] * reps)[:n]).cuda())
 
 
-def set_check(sm, on):
-    sm.set_left_right_check(1.0 if on else None)
+STATES = ("off", "on", "fill")   # no check, check, check + background fill
+
+
+def set_check(sm, state):
+    sm.set_left_right_check(None if state == "off" else 1.0, background_fill=state == "fill")
 
 
 def batch_leg(name, frames, iters):
@@ -65,23 +69,24 @@ def batch_leg(name, frames, iters):
     L, R = inputs(H, W, D, frames)
     out = torch.empty((frames, H, W), dtype=torch.float32, device="cuda")
     fn = lambda: sm.compute_disparity_batch(L, R, out)   # noqa: E731
-    res = {"off": [], "on": []}
-    for on in (False, True):   # warm-up of both paths
-        set_check(sm, on)
+    res = {s: [] for s in STATES}
+    for state in STATES:        # warm-up of every path
+        set_check(sm, state)
         for _ in range(3):
             fn()
     for _ in range(2):          # alternated
-        for on in (False, True):
-            set_check(sm, on)
-            res["on" if on else "off"].append(timed(fn, iters))
-    set_check(sm, True)
+        for state in STATES:
+            set_check(sm, state)
+            res[state].append(timed(fn, iters))
+    set_check(sm, "on")
     fn()
     invalid = float((out == -1.0).float().mean().item())
-    off, on = min(res["off"]), min(res["on"])
+    off, on, fill = min(res["off"]), min(res["on"]), min(res["fill"])
     return {"workload": name, "frames_per_step": frames, "frames_per_launch": sm.frames_per_launch,
-            "ms_per_step_off": off, "ms_per_step_on": on,
-            "frames_per_s_off": frames / off * 1e3, "frames_per_s_on": frames / on * 1e3, "on_over_off": on / off,
-            "invalid_fraction": invalid}
+            "ms_per_step_off": off, "ms_per_step_on": on, "ms_per_step_fill": fill,
+            "frames_per_s_off": frames / off * 1e3, "frames_per_s_on": frames / on * 1e3,
+            "frames_per_s_fill": frames / fill * 1e3, "on_over_off": on / off,
+            "fill_rate_over_check_rate": on / fill, "invalid_fraction": invalid}
 
 
 def single_frame_leg(name, iters=200):
@@ -92,16 +97,17 @@ def single_frame_leg(name, iters=200):
     l0, r0 = L[0].contiguous(), R[0].contiguous()
     fn = lambda: sm.compute_disparity_map(l0, r0)   # noqa: E731
     res = {}
-    for on in (False, True):
-        set_check(sm, on)
+    for state in STATES:
+        set_check(sm, state)
         for _ in range(10):
             fn()
     for _ in range(2):
-        for on in (False, True):
-            set_check(sm, on)
-            res.setdefault(on, []).append(timed(fn, iters))
-    return {"workload": name, "one_frame_per_call": True, "ms_per_frame_off": min(res[False]),
-            "ms_per_frame_on": min(res[True]), "on_over_off": min(res[True]) / min(res[False])}
+        for state in STATES:
+            set_check(sm, state)
+            res.setdefault(state, []).append(timed(fn, iters))
+    t = {s: min(v) for s, v in res.items()}
+    return {"workload": name, "one_frame_per_call": True, "ms_per_frame_off": t["off"], "ms_per_frame_on": t["on"],
+            "ms_per_frame_fill": t["fill"], "on_over_off": t["on"] / t["off"], "fill_over_on": t["fill"] / t["on"]}
 
 
 def profile_leg(name="C3", frames=64, iters=10):
@@ -111,8 +117,8 @@ def profile_leg(name="C3", frames=64, iters=10):
     L, R = inputs(H, W, D, frames)
     out = torch.empty((frames, H, W), dtype=torch.float32, device="cuda")
     res = {}
-    for on in (False, True):
-        set_check(sm, on)
+    for state in STATES:
+        set_check(sm, state)
         for _ in range(3):
             sm.compute_disparity_batch(L, R, out)
         torch.cuda.synchronize()
@@ -122,13 +128,14 @@ def profile_leg(name="C3", frames=64, iters=10):
             sm.compute_disparity_batch(L, R, out)
         d = sm.profile_read_detail()
         sm.profile(False)
-        res["on" if on else "off"] = {k: {"us_per_frame": ms * 1e3 / (frames * iters), "launches": n}
-                                      for k, (ms, n) in d.items()}
+        res[state] = {k: {"us_per_frame": ms * 1e3 / (frames * iters), "launches": n} for k, (ms, n) in d.items()}
     # kernel A with the check runs forward + mirrored frames in one launch: mirrored / forward = on / off - 1
     a_off, a_on = res["off"]["gray_pool"]["us_per_frame"], res["on"]["gray_pool"]["us_per_frame"]
     f_off, f_on = res["off"]["fill"]["us_per_frame"], res["on"]["fill"]["us_per_frame"]
     res["derived"] = {"mirrored_over_forward_kernel_a": a_on / a_off - 1.0,
-                      "fill_plus_check_minus_plain_fill_us_per_frame": f_on - 2.0 * f_off}
+                      "fill_plus_check_minus_plain_fill_us_per_frame": f_on - 2.0 * f_off,
+                      "fill_bucket_background_fill_minus_check_us_per_frame":
+                          res["fill"]["fill"]["us_per_frame"] - f_on}
     return {"workload": name, "frames_per_step": frames, "per_kernel": res}
 
 
@@ -141,16 +148,17 @@ def host_leg(name="C3", frames=64):
     out = torch.empty((frames, H, W), dtype=torch.float32).pin_memory()
     fn = lambda: sm.compute_disparity_host(Lh, Rh, out)   # noqa: E731
     res = {}
-    for on in (False, True):
-        set_check(sm, on)
+    for state in STATES:
+        set_check(sm, state)
         fn()
     for _ in range(2):
-        for on in (False, True):
-            set_check(sm, on)
-            res.setdefault(on, []).append(timed(fn, 2))
-    return {"workload": name, "host_path": True, "frames_per_call": frames,
-            "frames_per_s_off": frames / min(res[False]) * 1e3, "frames_per_s_on": frames / min(res[True]) * 1e3,
-            "on_over_off": min(res[True]) / min(res[False])}
+        for state in STATES:
+            set_check(sm, state)
+            res.setdefault(state, []).append(timed(fn, 2))
+    t = {s: min(v) for s, v in res.items()}
+    return {"workload": name, "host_path": True, "frames_per_call": frames, "frames_per_s_off": frames / t["off"] * 1e3,
+            "frames_per_s_on": frames / t["on"] * 1e3, "frames_per_s_fill": frames / t["fill"] * 1e3,
+            "on_over_off": t["on"] / t["off"], "fill_over_on": t["fill"] / t["on"]}
 
 
 def natural_leg():
@@ -166,19 +174,20 @@ def natural_leg():
         lt, rt = torch.from_numpy(l).cuda(), torch.from_numpy(r).cuda()
         fn = lambda: sm.compute_disparity_map(lt, rt)   # noqa: E731
         res = {}
-        for on in (False, True):
-            set_check(sm, on)
+        for state in STATES:
+            set_check(sm, state)
             for _ in range(5):
                 fn()
         for _ in range(2):
-            for on in (False, True):
-                set_check(sm, on)
-                res.setdefault(on, []).append(timed(fn, 50))
-        set_check(sm, True)
+            for state in STATES:
+                set_check(sm, state)
+                res.setdefault(state, []).append(timed(fn, 50))
+        set_check(sm, "on")
         inv = float((fn() == -1.0).float().mean().item())
-        rows.append({"natural_pair": f"{W}x{H} {mn}..{mx}", "ms_per_frame_off": min(res[False]),
-                     "ms_per_frame_on": min(res[True]), "on_over_off": min(res[True]) / min(res[False]),
-                     "invalid_fraction": inv})
+        t = {s: min(v) for s, v in res.items()}
+        rows.append({"natural_pair": f"{W}x{H} {mn}..{mx}", "ms_per_frame_off": t["off"], "ms_per_frame_on": t["on"],
+                     "ms_per_frame_fill": t["fill"], "on_over_off": t["on"] / t["off"],
+                     "fill_over_on": t["fill"] / t["on"], "invalid_fraction": inv})
     return rows
 
 
