@@ -6,6 +6,7 @@
 
 #include <stdlib.h>
 
+#include <memory>
 #include <new>
 #include <utility>
 #include <vector>
@@ -23,68 +24,151 @@ constexpr int kScreenPause = 32;        // chunks without the screen before it i
 constexpr size_t kGuardBytes = 64 << 10;  // per side, debug guard bands
 constexpr unsigned char kGuardPattern = 0xA5;
 constexpr int kProfMarks = 7;  // start | gray+pool | plane padding | level screen | cost+agg+WTA | secondary | fill
-}
+
+// Base of the resource owners below: a copy would free the same resources twice.
+struct NoCopy {
+    NoCopy() = default;
+    NoCopy(const NoCopy &) = delete;
+    NoCopy &operator=(const NoCopy &) = delete;
+};
+
+// The handle's device scratch: every live allocation as (raw base, payload bytes); the destructor frees what is left.
+// With debug guard bands (SD_DEBUG_GUARDS=1 at sd_create) every payload is bracketed by kGuardBytes of a known pattern;
+// sd_check_guards counts the bytes a stray store has changed (stands in for compute-sanitizer).
+struct DeviceAllocs : NoCopy {
+    bool guards = false;
+    std::vector<std::pair<char *, size_t>> live;
+    ~DeviceAllocs() { for (const auto &a : live) cudaFree(a.first); }
+
+    template <typename T>
+    cudaError_t alloc(T **p, size_t bytes) {
+        const size_t total = guards ? ((bytes + 255) & ~(size_t)255) + 2 * kGuardBytes : bytes;
+        char *raw = nullptr;
+        cudaError_t e = cudaMalloc((void **)&raw, total);
+        if (e != cudaSuccess) return e;
+        live.push_back(std::make_pair(raw, bytes));
+        if (guards && (e = cudaMemset(raw, kGuardPattern, total)) != cudaSuccess) return e;
+        *p = (T *)(raw + (guards ? kGuardBytes : 0));
+        return cudaSuccess;
+    }
+
+    // frees the allocation whose payload is p and sets p to null (no-op for null)
+    template <typename T>
+    void release(T *&p) {
+        for (size_t i = 0; p && i < live.size(); i++)
+            if (live[i].first + (guards ? kGuardBytes : 0) == (char *)p) {
+                cudaFree(live[i].first);
+                live.erase(live.begin() + i);
+                break;
+            }
+        p = nullptr;
+    }
+};
+
+// Streams, per-slot events and device slots of the pipelined host path (sd_compute_host) for one input dtype.  Every
+// member starts null and the destructor frees whatever was created, so a construction that fails partway leaks nothing.
+struct HostPipeline : NoCopy {
+    int dtype = -1;
+    cudaStream_t st_h2d = nullptr, st_comp = nullptr, st_d2h = nullptr;
+    void *din_l[kSlots] = {}, *din_r[kSlots] = {};
+    float *dout[kSlots] = {};
+    cudaEvent_t ev_h2d[kSlots] = {}, ev_comp[kSlots] = {}, ev_d2h[kSlots] = {};
+    ~HostPipeline() {
+        // (destroying a null event or stream would leave an error behind for the next cudaGetLastError)
+        for (int i = 0; i < kSlots; i++) {
+            cudaFree(din_l[i]);
+            cudaFree(din_r[i]);
+            cudaFree(dout[i]);
+            for (cudaEvent_t e : {ev_h2d[i], ev_comp[i], ev_d2h[i]})
+                if (e) cudaEventDestroy(e);
+        }
+        for (cudaStream_t s : {st_h2d, st_comp, st_d2h})
+            if (s) cudaStreamDestroy(s);
+    }
+};
+
+// A pinned host word mapped into the device's address space: kernels post to `dev`, the host reads `host`.
+struct MappedWord : NoCopy {
+    unsigned long long *host = nullptr, *dev = nullptr;
+    ~MappedWord() { if (host) cudaFreeHost(host); }
+
+    cudaError_t alloc() {
+        cudaError_t e = cudaHostAlloc((void **)&host, sizeof(*host), cudaHostAllocMapped);
+        if (e != cudaSuccess) {
+            host = nullptr;
+            return e;
+        }
+        *host = 0;
+        if ((e = cudaHostGetDevicePointer((void **)&dev, host, 0)) != cudaSuccess) dev = nullptr;
+        return e;
+    }
+};
+}  // namespace
 
 struct sd_handle {
-    sd_config cfg;
-    Geom g;
-    int device;
-    int chunk;       // frames per launch
-    int variant;     // 0 auto, 1 generic, 2 specialised, 3 warp-specialised
-    bool auto_ws;    // variant 0 picks the warp-specialised schedule for this shape (sd_create's cost model)
-    int sms, per_sm_fast;  // SM count and resident blocks per SM of the specialised kernel (launch cost models)
-    bool screen;     // certified level screen in front of the specialised kernel (default on where supported)
-    int epoch;       // chunk counter, tags the out-of-range flag of the screen
-    size_t parts_capacity;  // pixels the part slots of a level-split launch can hold (Scratch::wta4_parts)
-    bool split_off;  // sd_set_level_split(h, 0): never split (tuning / tests)
-    int abs_mode;    // layout of Scratch::agg_vol for the chunk in flight: 0 none, 1 whole volume, 2 compact (gather pass)
+    sd_config cfg = {};
+    Geom g = {};
+    int device = 0;
+    int chunk = 0;         // frames per launch
+    int variant = 0;       // 0 auto, 1 generic, 2 specialised, 3 warp-specialised
+    bool auto_ws = false;  // variant 0 picks the warp-specialised schedule for this shape (sd_create's cost model)
+    int sms = 0, per_sm_fast = 0;  // SM count and resident blocks per SM of the specialised kernel (launch cost models)
+    bool screen = false;   // certified level screen in front of the specialised kernel (default on where supported)
+    int epoch = 0;         // chunk counter, tags the out-of-range flag of the screen
+    size_t parts_capacity = 0;  // pixels the part slots of a level-split launch can hold (Scratch::wta4_parts)
+    bool split_off = false;     // sd_set_level_split(h, 0): never split (tuning / tests)
+    int abs_mode = 0;      // layout of Scratch::agg_vol for the chunk in flight: 0 none, 1 whole volume, 2 compact (gather pass)
     // Adaptive policy: the screen only pays off when it removes work.  The last block of every screen launch posts
     // {chunk tag, pairs screened, pairs flagged} as one 64-bit store to mapped host memory (no copy, no wait); the
     // next chunks look at the latest word that has arrived: if the fused kernel still had to evaluate more than
     // kScreenGiveUp of the level pairs, the screen is skipped for kScreenPause chunks and then probed again.
     // Results never depend on this -- the screen only changes the run time.
-    unsigned long long *stats_host;   // mapped pinned word
-    unsigned long long stats_seen;
-    int screen_pause;
-    Scratch s;
-    float *dbg_cost, *dbg_agg;
-    GrayView gv;     // band mode: where the left gray of the global image lives, else all zero
+    MappedWord stats;      // (its device alias is Scratch::screen_host_word)
+    unsigned long long stats_seen = 0;
+    int screen_pause = 0;
+    DeviceAllocs allocs;   // owns every device buffer of `s`, rmap and lr_rows
+    Scratch s = {};
+    float *dbg_cost = nullptr, *dbg_agg = nullptr;
+    GrayView gv = {};      // band mode: where the left gray of the global image lives, else all zero
     // peer-memory row bands (sd_band_p2p_*): one exported allocation per rank = [window L | window R | gray 0 | gray 1 | flags]
-    struct P2P {
-        bool on, connected;
-        int world, rank, dtype, halo_rows;
-        int row0[9];                 // full-resolution first row of every rank's band (+ total height)
-        size_t win_bytes, gray_bytes;  // per window / per published gray buffer (sized for the tallest band)
-        char *base;                  // my allocation
-        char *peer[8];               // every rank's allocation (peer[rank] == base)
-        unsigned epoch;
-        unsigned long long *timeout_host, *timeout_dev;   // mapped word a wait kernel posts {epoch, flag} to when a peer never shows up
+    struct P2P : NoCopy {
+        bool on = false, connected = false;
+        int world = 0, rank = 0, dtype = 0, halo_rows = 0;
+        int row0[9] = {};            // full-resolution first row of every rank's band (+ total height)
+        size_t win_bytes = 0, gray_bytes = 0;  // per window / per published gray buffer (sized for the tallest band)
+        char *base = nullptr;        // my allocation
+        char *peer[8] = {};          // every rank's allocation (peer[rank] == base)
+        unsigned epoch = 0;
+        MappedWord timeout;          // a wait kernel posts {epoch, flag} here when a peer never shows up
+        ~P2P() { close(); }
+        void close() {   // unmaps the peers' allocations and frees my own
+            for (int q = 0; q < world; q++)
+                if (q != rank && peer[q]) cudaIpcCloseMemHandle(peer[q]);
+            cudaFree(base);
+            base = nullptr;
+        }
     } p2p;
-    // host pipeline (lazily created by sd_compute_host)
-    bool host_ready;
-    int host_dtype;
-    cudaStream_t st_h2d, st_comp, st_d2h;
-    void *din_l[kSlots], *din_r[kSlots];
-    float *dout[kSlots];
-    cudaEvent_t ev_h2d[kSlots], ev_comp[kSlots], ev_d2h[kSlots];
+    std::unique_ptr<HostPipeline> host;   // lazily created by sd_compute_host
     // scratch is shared by every call on this handle: each call's stream first waits for the previous call's work
-    cudaEvent_t ev_last;
-    bool ev_last_valid;
+    cudaEvent_t ev_last = nullptr;
+    bool ev_last_valid = false;
     // optional per-kernel timing (sd_profile_enable): kProfMarks events per chunk on the launching stream
-    bool prof;
-    std::vector<cudaEvent_t> *prof_events;
-    // debug guard bands (SD_DEBUG_GUARDS=1 at sd_create): every scratch allocation is bracketed by kGuardBytes of a
-    // known pattern; sd_check_guards counts the bytes a stray store has changed (stands in for compute-sanitizer)
-    bool guards;
-    std::vector<std::pair<char *, size_t>> *guard_allocs;   // (raw base, payload bytes)
+    bool prof = false;
+    std::vector<cudaEvent_t> prof_events;
     // left-right consistency check (sd_set_lr_check): a chunk holds chunk/2 frame PAIRS, each run forward and mirrored
-    bool lr;
-    float lr_tol, lr_invalid;
-    float *rmap;     // [chunk/2][H][W] right views' disparity maps of the last chunk, in mirrored orientation
-    bool lr_fill;    // background fill of the rejected pixels (sd_set_lr_fill)
-    unsigned char *lr_rows;   // [chunk/2][H] per row: 1 if the check kept a pixel of it (the fill's column pass)
-    char err[640];
-    int last_cuda;
+    bool lr = false;
+    float lr_tol = 0.f, lr_invalid = 0.f;
+    float *rmap = nullptr;       // [chunk/2][H][W] right views' disparity maps of the last chunk, in mirrored orientation
+    bool lr_fill = false;        // background fill of the rejected pixels (sd_set_lr_fill)
+    unsigned char *lr_rows = nullptr;   // [chunk/2][H] per row: 1 if the check kept a pixel of it (the fill's column pass)
+    char err[640] = {};
+    int last_cuda = 0;
+
+    // (the members' destructors free the rest; sd_destroy runs this on the handle's device)
+    ~sd_handle() {
+        for (cudaEvent_t e : prof_events) cudaEventDestroy(e);
+        if (ev_last) cudaEventDestroy(ev_last);
+    }
 };
 
 namespace {
@@ -120,33 +204,6 @@ struct DeviceGuard {
         if (prev >= 0 && cudaGetDevice(&cur) == cudaSuccess && cur != prev) cudaSetDevice(prev);
     }
 };
-
-// Scratch allocation: plain cudaMalloc, or (debug) payload bracketed by two guard bands filled with kGuardPattern.
-cudaError_t scratch_alloc(sd_handle *h, void **p, size_t bytes) {
-    if (!h->guards) return cudaMalloc(p, bytes);
-    const size_t padded = (bytes + 255) & ~(size_t)255;
-    char *raw = nullptr;
-    cudaError_t e = cudaMalloc((void **)&raw, padded + 2 * kGuardBytes);
-    if (e != cudaSuccess) return e;
-    e = cudaMemset(raw, kGuardPattern, padded + 2 * kGuardBytes);
-    if (e != cudaSuccess) return e;
-    h->guard_allocs->push_back(std::make_pair(raw, bytes));
-    *p = raw + kGuardBytes;
-    return cudaSuccess;
-}
-
-void scratch_free(sd_handle *h, void *p) {
-    if (!p) return;
-    if (h->guards && h->guard_allocs) {
-        for (auto &a : *h->guard_allocs)
-            if (a.first + kGuardBytes == (char *)p) {
-                cudaFree(a.first);
-                a.first = nullptr;
-                return;
-            }
-    }
-    cudaFree(p);
-}
 
 const char *validate(const sd_config *c) {
     if (c->height <= 0 || c->width <= 0) return "height and width must be positive";
@@ -204,8 +261,8 @@ int prof_mark(sd_handle *h, cudaStream_t st) {
     if (!h->prof) return SD_OK;
     cudaEvent_t e;
     SD_CUDA(h, cudaEventCreate(&e));
+    h->prof_events.push_back(e);
     SD_CUDA(h, cudaEventRecord(e, st));
-    h->prof_events->push_back(e);
     return SD_OK;
 }
 
@@ -325,8 +382,8 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
         h->s.range_epoch = ++h->epoch;
         const int v = active_variant(h, frames);
         bool screen = (v == 2) && screen_active(h, frames);
-        if (screen && h->stats_host) {
-            const unsigned long long w = *(volatile unsigned long long *)h->stats_host;   // [tag:16][screened:24][flagged:24]
+        if (screen && h->stats.host) {
+            const unsigned long long w = *(volatile unsigned long long *)h->stats.host;   // [tag:16][screened:24][flagged:24]
             if (w != h->stats_seen) {
                 const double flagged = (double)(w & 0xffffffull), screened = (double)((w >> 24) & 0xffffffull);
                 const double give_up = h->s.agg_vol ? kScreenGiveUpGather : kScreenGiveUp;
@@ -389,22 +446,6 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
     return SD_OK;
 }
 
-void destroy_host_pipeline(sd_handle *h) {
-    if (!h->host_ready) return;
-    for (int i = 0; i < kSlots; i++) {
-        cudaFree(h->din_l[i]);
-        cudaFree(h->din_r[i]);
-        cudaFree(h->dout[i]);
-        cudaEventDestroy(h->ev_h2d[i]);
-        cudaEventDestroy(h->ev_comp[i]);
-        cudaEventDestroy(h->ev_d2h[i]);
-    }
-    cudaStreamDestroy(h->st_h2d);
-    cudaStreamDestroy(h->st_comp);
-    cudaStreamDestroy(h->st_d2h);
-    h->host_ready = false;
-}
-
 // Frames per chunk of the pipelined host path: copies of a chunk cannot overlap its own kernels, so the host path uses
 // chunks of at most 8 frames whatever the device path's chunk is (SD_HOST_CHUNK: tuning knob).
 int host_chunk(const sd_handle *h) {
@@ -420,26 +461,25 @@ int host_chunk_frames(const sd_handle *h) {
 }
 
 int ensure_host_pipeline(sd_handle *h, int dtype) {
-    if (h->host_ready && h->host_dtype == dtype) return SD_OK;
-    destroy_host_pipeline(h);
+    if (h->host && h->host->dtype == dtype) return SD_OK;
+    h->host.reset();
+    std::unique_ptr<HostPipeline> p(new (std::nothrow) HostPipeline());
+    if (!p) return fail(h, SD_ERR_NOMEM, "out of host memory");
     const size_t inb = in_bytes_per_frame(h, dtype) * host_chunk(h);
     const size_t outb = (size_t)h->g.H * h->g.W * sizeof(float) * host_chunk(h);
-    memset(h->din_l, 0, sizeof(h->din_l));
-    memset(h->din_r, 0, sizeof(h->din_r));
-    memset(h->dout, 0, sizeof(h->dout));
-    SD_CUDA(h, cudaStreamCreateWithFlags(&h->st_h2d, cudaStreamNonBlocking));
-    SD_CUDA(h, cudaStreamCreateWithFlags(&h->st_comp, cudaStreamNonBlocking));
-    SD_CUDA(h, cudaStreamCreateWithFlags(&h->st_d2h, cudaStreamNonBlocking));
+    SD_CUDA(h, cudaStreamCreateWithFlags(&p->st_h2d, cudaStreamNonBlocking));
+    SD_CUDA(h, cudaStreamCreateWithFlags(&p->st_comp, cudaStreamNonBlocking));
+    SD_CUDA(h, cudaStreamCreateWithFlags(&p->st_d2h, cudaStreamNonBlocking));
     for (int i = 0; i < kSlots; i++) {
-        SD_CUDA(h, cudaMalloc(&h->din_l[i], inb));
-        SD_CUDA(h, cudaMalloc(&h->din_r[i], inb));
-        SD_CUDA(h, cudaMalloc((void **)&h->dout[i], outb));
-        SD_CUDA(h, cudaEventCreateWithFlags(&h->ev_h2d[i], cudaEventDisableTiming));
-        SD_CUDA(h, cudaEventCreateWithFlags(&h->ev_comp[i], cudaEventDisableTiming));
-        SD_CUDA(h, cudaEventCreateWithFlags(&h->ev_d2h[i], cudaEventDisableTiming));
+        SD_CUDA(h, cudaMalloc(&p->din_l[i], inb));
+        SD_CUDA(h, cudaMalloc(&p->din_r[i], inb));
+        SD_CUDA(h, cudaMalloc((void **)&p->dout[i], outb));
+        SD_CUDA(h, cudaEventCreateWithFlags(&p->ev_h2d[i], cudaEventDisableTiming));
+        SD_CUDA(h, cudaEventCreateWithFlags(&p->ev_comp[i], cudaEventDisableTiming));
+        SD_CUDA(h, cudaEventCreateWithFlags(&p->ev_d2h[i], cudaEventDisableTiming));
     }
-    h->host_ready = true;
-    h->host_dtype = dtype;
+    p->dtype = dtype;
+    h->host = std::move(p);
     return SD_OK;
 }
 
@@ -472,14 +512,10 @@ int sd_create(const sd_config *cfg, int device, int frames_per_launch, sd_handle
     *out = nullptr;
     sd_handle *h = new (std::nothrow) sd_handle();
     if (!h) return SD_ERR_NOMEM;
-    memset(h, 0, sizeof(*h));
     *out = h;  // returned even on failure so the caller can read sd_last_error, then sd_destroy
-    h->prof_events = new (std::nothrow) std::vector<cudaEvent_t>();
-    h->guard_allocs = new (std::nothrow) std::vector<std::pair<char *, size_t>>();
-    if (!h->prof_events || !h->guard_allocs) return fail(h, SD_ERR_NOMEM, "out of host memory");
     {
         const char *e = getenv("SD_DEBUG_GUARDS");
-        h->guards = e && atoi(e) != 0;
+        h->allocs.guards = e && atoi(e) != 0;
     }
     h->cfg = *cfg;
     h->device = device;
@@ -545,16 +581,16 @@ int sd_create(const sd_config *cfg, int device, int frames_per_launch, sd_handle
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     SD_CUDA(h, cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming));
     const size_t F = h->chunk, n = (size_t)g.H * g.W, nd = (size_t)g.Hd * g.Wd;
-    SD_CUDA(h, scratch_alloc(h, (void **)&h->s.gray, F * 2 * n * sizeof(float)));
-    SD_CUDA(h, scratch_alloc(h, (void **)&h->s.pool, F * 2 * nd * sizeof(float)));
-    SD_CUDA(h, scratch_alloc(h, (void **)&h->s.wta4, F * nd * sizeof(float4)));
-    SD_CUDA(h, scratch_alloc(h, (void **)&h->s.edge2, F * nd * sizeof(float2)));
-    SD_CUDA(h, scratch_alloc(h, (void **)&h->s.refined, F * nd * sizeof(float)));
+    SD_CUDA(h, h->allocs.alloc(&h->s.gray, F * 2 * n * sizeof(float)));
+    SD_CUDA(h, h->allocs.alloc(&h->s.pool, F * 2 * nd * sizeof(float)));
+    SD_CUDA(h, h->allocs.alloc(&h->s.wta4, F * nd * sizeof(float4)));
+    SD_CUDA(h, h->allocs.alloc(&h->s.edge2, F * nd * sizeof(float2)));
+    SD_CUDA(h, h->allocs.alloc(&h->s.refined, F * nd * sizeof(float)));
     if (mbm_wta_fast_supported(g)) {
         const PadGeom pg = make_pad_geom(g.Hd, g.Wd, g.L, g.min_ds);
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->s.padl, F * (size_t)pg.rows * pg.pwl * sizeof(float)));
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->s.padr, F * (size_t)pg.rows * pg.pwr * sizeof(float)));
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->s.range_flag, sizeof(int)));
+        SD_CUDA(h, h->allocs.alloc(&h->s.padl, F * (size_t)pg.rows * pg.pwl * sizeof(float)));
+        SD_CUDA(h, h->allocs.alloc(&h->s.padr, F * (size_t)pg.rows * pg.pwr * sizeof(float)));
+        SD_CUDA(h, h->allocs.alloc(&h->s.range_flag, sizeof(int)));
         SD_CUDA(h, cudaMemset(h->s.range_flag, 0, sizeof(int)));
         {   // part slots for level-split launches: sized for the largest split any launch size of this handle would pick
             // (unscreened: plan_split; behind the screen: up to 8 parts while the launch has fewer than four waves of tiles)
@@ -573,22 +609,21 @@ int sd_create(const sd_config *cfg, int device, int frames_per_launch, sd_handle
                 if (S > 1 && (size_t)S * f * nd > need) need = (size_t)S * f * nd;
             }
             if (need > 0 && need * (sizeof(float4) + sizeof(float2)) <= ((size_t)1 << 30)) {
-                SD_CUDA(h, scratch_alloc(h, (void **)&h->s.wta4_parts, need * sizeof(float4)));
-                SD_CUDA(h, scratch_alloc(h, (void **)&h->s.edge2_parts, need * sizeof(float2)));
-                SD_CUDA(h, scratch_alloc(h, (void **)&h->s.part_range, (size_t)kMaxSplit * F * tiles1 * sizeof(int2)));
+                SD_CUDA(h, h->allocs.alloc(&h->s.wta4_parts, need * sizeof(float4)));
+                SD_CUDA(h, h->allocs.alloc(&h->s.edge2_parts, need * sizeof(float2)));
+                SD_CUDA(h, h->allocs.alloc(&h->s.part_range, (size_t)kMaxSplit * F * tiles1 * sizeof(int2)));
                 h->parts_capacity = need;
             }
         }
         if (mbm_screen_supported(g)) {
-            SD_CUDA(h, scratch_alloc(h, (void **)&h->s.pass_mask, F * (size_t)pg.tiles_x * pg.tiles_y * 4 * sizeof(unsigned)));
-            SD_CUDA(h, scratch_alloc(h, (void **)&h->s.gather_mask, F * (size_t)pg.tiles_x * pg.tiles_y * 4 * sizeof(unsigned)));
-            SD_CUDA(h, scratch_alloc(h, (void **)&h->s.tile_order, F * (size_t)pg.tiles_x * pg.tiles_y * kScreenBuckets * sizeof(int)));
-            SD_CUDA(h, scratch_alloc(h, (void **)&h->s.bucket_count, kScreenCtrlInts * sizeof(int)));
-            SD_CUDA(h, scratch_alloc(h, (void **)&h->s.screen_stats, 2 * sizeof(unsigned long long)));
+            SD_CUDA(h, h->allocs.alloc(&h->s.pass_mask, F * (size_t)pg.tiles_x * pg.tiles_y * 4 * sizeof(unsigned)));
+            SD_CUDA(h, h->allocs.alloc(&h->s.gather_mask, F * (size_t)pg.tiles_x * pg.tiles_y * 4 * sizeof(unsigned)));
+            SD_CUDA(h, h->allocs.alloc(&h->s.tile_order, F * (size_t)pg.tiles_x * pg.tiles_y * kScreenBuckets * sizeof(int)));
+            SD_CUDA(h, h->allocs.alloc(&h->s.bucket_count, kScreenCtrlInts * sizeof(int)));
+            SD_CUDA(h, h->allocs.alloc(&h->s.screen_stats, 2 * sizeof(unsigned long long)));
             SD_CUDA(h, cudaMemset(h->s.screen_stats, 0, 2 * sizeof(unsigned long long)));
-            SD_CUDA(h, cudaHostAlloc((void **)&h->stats_host, sizeof(unsigned long long), cudaHostAllocMapped));
-            *h->stats_host = 0;
-            SD_CUDA(h, cudaHostGetDevicePointer((void **)&h->s.screen_host_word, h->stats_host, 0));
+            SD_CUDA(h, h->stats.alloc());
+            h->s.screen_host_word = h->stats.dev;
             h->screen = true;
         }
     }
@@ -606,10 +641,9 @@ int sd_set_compat(sd_handle *h, int on) {
         // sized for both layouts: the whole volume [L][Hd*Wd] and the compact per-tile one of the gather pass
         size_t per_frame = (size_t)h->g.Hd * h->g.Wd * h->g.L;
         if (h->s.gather_mask && compact_volume_floats(h->g) > per_frame) per_frame = compact_volume_floats(h->g);
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->s.agg_vol, (size_t)h->chunk * per_frame * sizeof(float)));
-    } else if (!on && h->s.agg_vol) {
-        scratch_free(h, h->s.agg_vol);
-        h->s.agg_vol = nullptr;
+        SD_CUDA(h, h->allocs.alloc(&h->s.agg_vol, (size_t)h->chunk * per_frame * sizeof(float)));
+    } else if (!on) {
+        h->allocs.release(h->s.agg_vol);
     }
     h->g.abs_index = on ? 1 : 0;
     return SD_OK;
@@ -619,48 +653,13 @@ int sd_check_guards(sd_handle *h, long long *corrupted_bytes);
 
 int sd_destroy(sd_handle *h) {
     if (!h) return SD_OK;
-    if (h->guards && h->guard_allocs && !h->guard_allocs->empty()) {
+    if (h->allocs.guards && !h->allocs.live.empty()) {
         // debug handles (SD_DEBUG_GUARDS=1) check their guard bands one last time: a whole test run can be soaked this way
         long long bad = 0;
         if (sd_check_guards(h, &bad) == SD_OK && bad != 0)
             fprintf(stderr, "libstereo_b200: GUARD BANDS CORRUPTED: %lld bytes around the scratch of a %dx%d handle\n", bad, h->g.H, h->g.W);
     }
-    {
-        DeviceGuard dg(h->device);
-        destroy_host_pipeline(h);
-        scratch_free(h, h->s.gray);
-        scratch_free(h, h->s.pool);
-        scratch_free(h, h->s.wta4);
-        scratch_free(h, h->s.edge2);
-        scratch_free(h, h->s.refined);
-        scratch_free(h, h->s.wta4_parts);
-        scratch_free(h, h->s.edge2_parts);
-        scratch_free(h, h->s.part_range);
-        if (h->ev_last) cudaEventDestroy(h->ev_last);
-        scratch_free(h, h->s.agg_vol);
-        scratch_free(h, h->s.padl);
-        scratch_free(h, h->s.padr);
-        if (h->p2p.on) {
-            for (int q = 0; q < h->p2p.world; q++)
-                if (q != h->p2p.rank && h->p2p.peer[q]) cudaIpcCloseMemHandle(h->p2p.peer[q]);
-            cudaFree(h->p2p.base);
-            if (h->p2p.timeout_host) cudaFreeHost(h->p2p.timeout_host);
-        }
-        if (h->stats_host) cudaFreeHost(h->stats_host);
-        scratch_free(h, h->s.pass_mask);
-        scratch_free(h, h->s.gather_mask);
-        scratch_free(h, h->s.tile_order);
-        scratch_free(h, h->s.bucket_count);
-        scratch_free(h, h->s.screen_stats);
-        scratch_free(h, h->s.range_flag);
-        scratch_free(h, h->rmap);
-        scratch_free(h, h->lr_rows);
-        if (h->prof_events) {
-            for (cudaEvent_t e : *h->prof_events) cudaEventDestroy(e);
-            delete h->prof_events;
-        }
-        delete h->guard_allocs;
-    }
+    DeviceGuard dg(h->device);
     delete h;
     return SD_OK;
 }
@@ -763,8 +762,7 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     if (g.H != band_row0[rank + 1] - band_row0[rank] + 2 * halo_rows) return fail(h, SD_ERR_SHAPE, "the handle's height must be band rows + 2 * halo rows");
     DeviceGuard dg(h->device);
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
-    sd_handle::P2P &p = h->p2p;
-    memset(&p, 0, sizeof(p));
+    sd_handle::P2P &p = h->p2p;   // (as created: an init that failed has closed it again)
     p.world = world;
     p.rank = rank;
     p.dtype = dtype;
@@ -779,15 +777,11 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     if (e == cudaSuccess) e = cudaDeviceSynchronize();
     if (e == cudaSuccess) e = cudaIpcGetMemHandle(&ipc, p.base);
     if (e != cudaSuccess) {
-        cudaFree(p.base);
-        p.base = nullptr;
+        p.close();
         return fail_cuda(h, e, "sd_band_p2p_init (memset / cudaIpcGetMemHandle)");
     }
     p.peer[rank] = p.base;
-    if (cudaHostAlloc((void **)&p.timeout_host, sizeof(unsigned long long), cudaHostAllocMapped) == cudaSuccess) {
-        *p.timeout_host = 0;
-        if (cudaHostGetDevicePointer((void **)&p.timeout_dev, p.timeout_host, 0) != cudaSuccess) p.timeout_dev = nullptr;
-    }
+    p.timeout.alloc();   // optional: without it a peer that never shows up is not reported
     static_assert(sizeof(ipc) == 64, "cudaIpcMemHandle_t is 64 bytes");
     memcpy(ipc_handle_out, &ipc, sizeof(ipc));
     p.on = true;
@@ -817,8 +811,8 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
     sd_handle::P2P &p = h->p2p;
     if (!p.on || !p.connected) return fail(h, SD_ERR_BAD_ARG, "peer-memory band mode is not connected (sd_band_p2p_init / _connect)");
     if (h->chunk < 1) return fail(h, SD_ERR_SHAPE, "handle has no scratch");
-    if (p.timeout_host && *(volatile unsigned long long *)p.timeout_host != 0) {
-        const unsigned long long w = *(volatile unsigned long long *)p.timeout_host;
+    if (p.timeout.host && *(volatile unsigned long long *)p.timeout.host != 0) {
+        const unsigned long long w = *(volatile unsigned long long *)p.timeout.host;
         snprintf(h->err, sizeof(h->err), "row-band exchange timed out: frame %llu never received flag %llu from a peer rank "
                  "(a rank failed or made fewer sd_band_p2p_compute calls); results since then are invalid", w >> 32, (w & 0xffffffffull) - 1);
         return SD_ERR_CUDA;
@@ -841,7 +835,7 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
                                    halo, band_rows + 2 * halo, rows_of(prev) + 2 * halo, rows_of(next) + 2 * halo,
                                    myflags + kCtrScatter, p2p_flags(h, prev) + kFlagFromNext, p2p_flags(h, next) + kFlagFromPrev,
                                    epoch, st));
-    SD_CUDA(h, launch_wait_flags(myflags, kFlagFromPrev, 2, epoch, p.timeout_dev, st));
+    SD_CUDA(h, launch_wait_flags(myflags, kFlagFromPrev, 2, epoch, p.timeout.dev, st));
     // gray + pool on the local window [top halo | band | bottom halo]
     // (h->g is the handle's own geometry and is rewritten for the two halves of every frame: a handle is not
     //  thread-safe -- include/stereo_b200.h -- and the kernels receive Geom by value, so launches already in flight keep
@@ -858,7 +852,7 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
     for (int q = 0; q < n; q++) peer_flags[q] = p2p_flags(h, q) + kFlagGray + r;
     SD_CUDA(h, launch_publish_gray(h->s.gray + (size_t)halo * W, p2p_gray(h, r, parity), (size_t)band_rows * W,
                                    myflags + kCtrPublish, peer_flags, n, epoch, st));
-    SD_CUDA(h, launch_wait_flags(myflags, kFlagGray, n, epoch, p.timeout_dev, st));
+    SD_CUDA(h, launch_wait_flags(myflags, kFlagGray, n, epoch, p.timeout.dev, st));
     // matching + secondary + fill on the window; the fill reads its colour row from whichever rank owns it
     h->g.band_x_off = (p.row0[r] - halo) / g.K;
     h->g.H_glob = p.row0[n];
@@ -883,7 +877,8 @@ int sd_compute_host(sd_handle *h, const void *left, const void *right, int dtype
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     int rc = ensure_host_pipeline(h, dtype);
     if (rc != SD_OK) return rc;
-    rc = order_after_previous(h, h->st_comp);
+    const HostPipeline &hp = *h->host;
+    rc = order_after_previous(h, hp.st_comp);
     if (rc != SD_OK) return rc;
     const size_t inb = in_bytes_per_frame(h, dtype), outn = (size_t)h->g.H * h->g.W;
     // Chunk schedule: a short first chunk (its H2D copy cannot overlap anything) and a short last chunk (neither
@@ -896,15 +891,15 @@ int sd_compute_host(sd_handle *h, const void *left, const void *right, int dtype
     int it = 0;
     // On any failure below, copies to / from the caller's host buffers may still be in flight: drain before returning.
     struct Drain {
-        sd_handle *h;
+        const HostPipeline &hp;
         bool armed;
         ~Drain() {
             if (!armed) return;
-            cudaStreamSynchronize(h->st_h2d);
-            cudaStreamSynchronize(h->st_comp);
-            cudaStreamSynchronize(h->st_d2h);
+            cudaStreamSynchronize(hp.st_h2d);
+            cudaStreamSynchronize(hp.st_comp);
+            cudaStreamSynchronize(hp.st_d2h);
         }
-    } drain{h, true};
+    } drain{hp, true};
     for (int f0 = 0; f0 < n_frames; it++) {
         int nf = hc;
         const int left_over = n_frames - f0;
@@ -914,23 +909,23 @@ int sd_compute_host(sd_handle *h, const void *left, const void *right, int dtype
         if (nf > left_over) nf = left_over;
         const int sl = it % kSlots;
         // inputs of slot sl may be overwritten once the kernels of its previous use are done
-        if (it >= kSlots) SD_CUDA(h, cudaStreamWaitEvent(h->st_h2d, h->ev_comp[sl], 0));
-        SD_CUDA(h, cudaMemcpyAsync(h->din_l[sl], (const char *)left + inb * f0, inb * nf, cudaMemcpyHostToDevice, h->st_h2d));
-        SD_CUDA(h, cudaMemcpyAsync(h->din_r[sl], (const char *)right + inb * f0, inb * nf, cudaMemcpyHostToDevice, h->st_h2d));
-        SD_CUDA(h, cudaEventRecord(h->ev_h2d[sl], h->st_h2d));
-        SD_CUDA(h, cudaStreamWaitEvent(h->st_comp, h->ev_h2d[sl], 0));
+        if (it >= kSlots) SD_CUDA(h, cudaStreamWaitEvent(hp.st_h2d, hp.ev_comp[sl], 0));
+        SD_CUDA(h, cudaMemcpyAsync(hp.din_l[sl], (const char *)left + inb * f0, inb * nf, cudaMemcpyHostToDevice, hp.st_h2d));
+        SD_CUDA(h, cudaMemcpyAsync(hp.din_r[sl], (const char *)right + inb * f0, inb * nf, cudaMemcpyHostToDevice, hp.st_h2d));
+        SD_CUDA(h, cudaEventRecord(hp.ev_h2d[sl], hp.st_h2d));
+        SD_CUDA(h, cudaStreamWaitEvent(hp.st_comp, hp.ev_h2d[sl], 0));
         // the output of slot sl may be overwritten once its previous D2H is done
-        if (it >= kSlots) SD_CUDA(h, cudaStreamWaitEvent(h->st_comp, h->ev_d2h[sl], 0));
-        rc = run_chunk(h, h->din_l[sl], h->din_r[sl], dtype, nf, h->dout[sl], h->st_comp);
+        if (it >= kSlots) SD_CUDA(h, cudaStreamWaitEvent(hp.st_comp, hp.ev_d2h[sl], 0));
+        rc = run_chunk(h, hp.din_l[sl], hp.din_r[sl], dtype, nf, hp.dout[sl], hp.st_comp);
         if (rc != SD_OK) return rc;
-        SD_CUDA(h, cudaEventRecord(h->ev_comp[sl], h->st_comp));
-        SD_CUDA(h, cudaStreamWaitEvent(h->st_d2h, h->ev_comp[sl], 0));
-        SD_CUDA(h, cudaMemcpyAsync(out + outn * f0, h->dout[sl], outn * nf * sizeof(float), cudaMemcpyDeviceToHost, h->st_d2h));
-        SD_CUDA(h, cudaEventRecord(h->ev_d2h[sl], h->st_d2h));
+        SD_CUDA(h, cudaEventRecord(hp.ev_comp[sl], hp.st_comp));
+        SD_CUDA(h, cudaStreamWaitEvent(hp.st_d2h, hp.ev_comp[sl], 0));
+        SD_CUDA(h, cudaMemcpyAsync(out + outn * f0, hp.dout[sl], outn * nf * sizeof(float), cudaMemcpyDeviceToHost, hp.st_d2h));
+        SD_CUDA(h, cudaEventRecord(hp.ev_d2h[sl], hp.st_d2h));
         f0 += nf;
     }
-    SD_CUDA(h, cudaStreamSynchronize(h->st_d2h));
-    SD_CUDA(h, cudaStreamSynchronize(h->st_comp));
+    SD_CUDA(h, cudaStreamSynchronize(hp.st_d2h));
+    SD_CUDA(h, cudaStreamSynchronize(hp.st_comp));
     drain.armed = false;
     h->ev_last_valid = false;  // everything on this handle has completed
     return SD_OK;
@@ -1054,10 +1049,8 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
         if (h->rmap) {
             DeviceGuard dg(h->device);
             if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
-            scratch_free(h, h->rmap);
-            scratch_free(h, h->lr_rows);
-            h->rmap = nullptr;
-            h->lr_rows = nullptr;
+            h->allocs.release(h->rmap);
+            h->allocs.release(h->lr_rows);
         }
         h->lr = false;
         h->lr_fill = false;
@@ -1071,7 +1064,7 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
     if (!h->rmap) {
         DeviceGuard dg(h->device);
         if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->rmap, (size_t)lr_pairs(h) * h->g.H * h->g.W * sizeof(float)));
+        SD_CUDA(h, h->allocs.alloc(&h->rmap, (size_t)lr_pairs(h) * h->g.H * h->g.W * sizeof(float)));
     }
     h->lr = true;
     h->lr_tol = tolerance;
@@ -1085,7 +1078,7 @@ int sd_set_lr_fill(sd_handle *h, int on) {
     if (on && !h->lr_rows) {
         DeviceGuard dg(h->device);
         if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
-        SD_CUDA(h, scratch_alloc(h, (void **)&h->lr_rows, (size_t)lr_pairs(h) * h->g.H));
+        SD_CUDA(h, h->allocs.alloc(&h->lr_rows, (size_t)lr_pairs(h) * h->g.H));
     }
     h->lr_fill = on != 0;
     return SD_OK;
@@ -1154,7 +1147,7 @@ int sd_profile_enable(sd_handle *h, int on) {
 
 static int profile_collect(sd_handle *h, double *ms6, int *n6) {
     DeviceGuard dg(h->device);
-    std::vector<cudaEvent_t> &ev = *h->prof_events;
+    std::vector<cudaEvent_t> &ev = h->prof_events;
     for (int k = 0; k < kProfMarks - 1; k++) {
         ms6[k] = 0.0;
         n6[k] = 0;
@@ -1192,14 +1185,13 @@ int sd_profile_read_detail(sd_handle *h, double *ms, int *launches) {
 int sd_check_guards(sd_handle *h, long long *corrupted_bytes) {
     if (!h || !corrupted_bytes) return SD_ERR_BAD_ARG;
     *corrupted_bytes = 0;
-    if (!h->guards) return fail(h, SD_ERR_UNSUPPORTED, "guard bands are off: create the handle with SD_DEBUG_GUARDS=1 in the environment");
+    if (!h->allocs.guards) return fail(h, SD_ERR_UNSUPPORTED, "guard bands are off: create the handle with SD_DEBUG_GUARDS=1 in the environment");
     DeviceGuard dg(h->device);
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     SD_CUDA(h, cudaDeviceSynchronize());
     std::vector<unsigned char> host(kGuardBytes + 256);
     long long bad = 0;
-    for (const auto &a : *h->guard_allocs) {
-        if (!a.first) continue;
+    for (const auto &a : h->allocs.live) {
         const size_t padded = (a.second + 255) & ~(size_t)255;
         // front band; then [payload end, padded end) + back band
         SD_CUDA(h, cudaMemcpy(host.data(), a.first, kGuardBytes, cudaMemcpyDeviceToHost));
