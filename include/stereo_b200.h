@@ -215,6 +215,28 @@ int sd_set_lr_fill(sd_handle *h, int on);
 int sd_lr_fill(const float *left_map, const float *right_map, int n, int H, int W, float tolerance, float invalid_disparity,
                float *out, void *cuda_stream);
 
+/* Stereo rectification on the device, off by default: with it on, every entry point (sd_compute, sd_compute_host) takes
+ * RAW frames and first remaps each view exactly as cv2.remap(src, map_x, map_y, INTER_LINEAR, BORDER_CONSTANT, 0) with
+ * the CV_32FC1 maps of cv2.initUndistortRectifyMap (rule: DESIGN.md §14), then runs the unchanged pipeline on the
+ * rectified frames.  Source and rectified images are both the handle's H x W.
+ *   sd_set_rectification  the four maps: device float32 [H][W] each (output pixel -> source coordinate).  They are
+ *                         copied into the handle, stream-ordered on cuda_stream, so the caller may reuse or free theirs
+ *                         in that stream's order.  Allocates 4 * H * W floats of maps plus the rectified frames of one
+ *                         chunk, frames_per_launch * 2 * 3 * H * W * 4 bytes (sized for float32 input; 1.44 GB at the
+ *                         1080p default of 29 frames per launch).  All four maps NULL switches rectification off, frees
+ *                         both and restores the unrectified path exactly; a partial set of NULLs is SD_ERR_BAD_ARG.
+ *                         The remap is one more launch per chunk (sd_launches_per_call) and counts as kernel 0 in the
+ *                         per-kernel profile.  SD_ERR_UNSUPPORTED for H or W >= 32768 and together with the row-band
+ *                         modes (sd_set_band, sd_band_p2p_init, sd_compute_range), in either order.
+ *   sd_rectify            the same remap without a handle: n_planes [H][W] planes of dtype (SD_U8 / SD_F32) at src,
+ *                         each sampled with the same map, written to dst (device memory, must not overlap src).
+ *                         Asynchronous on cuda_stream.  SD_ERR_BAD_ARG for null pointers, non-positive sizes, H or
+ *                         W >= 32768, an unknown dtype or dst == src; SD_ERR_CUDA if the launch fails. */
+int sd_set_rectification(sd_handle *h, const float *left_map_x, const float *left_map_y, const float *right_map_x,
+                         const float *right_map_y, void *cuda_stream);
+int sd_rectify(const float *map_x, const float *map_y, const void *src, void *dst, int dtype, int n_planes, int H, int W,
+               void *cuda_stream);
+
 /* Level split for launches that cannot fill the GPU (one small frame, a thin row band): the unscreened specialised
  * kernel then spreads every tile's disparity levels over several blocks and a small kernel merges the partial
  * winner-take-all records (identical results: the maximum is taken in ascending level order with strict '>').

@@ -1,7 +1,8 @@
 """GPU versions of what the reference does with the disparity map after the hot path:
 accuracy metrics (depth_estimation_pipeline_metrics.py:18-56) and the point cloud
 (depth_estimation_pipeline_hooks.py:84-92, helpers/point_cloud_helpers.py:5-13); and the left-right check with the
-background fill for callers that hold both views' disparity maps."""
+background fill for callers that hold both views' disparity maps; and the rectification remap for callers that want
+a rectified image itself (to colour a point cloud or display a map)."""
 import math
 
 import torch
@@ -78,4 +79,36 @@ def left_right_fill(left_map: torch.Tensor, right_map: torch.Tensor, tolerance: 
     with torch.cuda.device(left_map.device):
         _check(N.lib().sd_lr_fill(left_map.data_ptr(), right_map.data_ptr(), n, H, W, tolerance,
                                   float(invalid_disparity), out.data_ptr(), stream), "sd_lr_fill")
+    return out
+
+
+def rectify(images: torch.Tensor, map_x: torch.Tensor, map_y: torch.Tensor, out=None):
+    """cv2.remap(image, map_x, map_y, cv2.INTER_LINEAR, borderMode=cv2.BORDER_CONSTANT, borderValue=0) of every [H,W]
+    plane of a [..., H, W] uint8 or float32 CUDA tensor (e.g. [3,H,W] CHW or [N,3,H,W]), bit for bit (DESIGN.md §14).
+    map_x / map_y: float32 [H,W] (cv2.initUndistortRectifyMap with m1type=cv2.CV_32FC1), on the images' device.
+    Returns `out` (a new tensor when None), which must not be `images`."""
+    if not all(isinstance(t, torch.Tensor) for t in (images, map_x, map_y)):
+        raise TypeError("images, map_x and map_y must be tensors")
+    if images.dim() < 2 or not images.is_cuda or images.dtype not in (torch.uint8, torch.float32):
+        raise RuntimeError("images must be a uint8 or float32 CUDA tensor of shape [..., H, W]")
+    H, W = images.shape[-2:]
+    for t, name in ((map_x, "map_x"), (map_y, "map_y")):
+        if t.dtype != torch.float32 or tuple(t.shape) != (H, W) or t.device != images.device:
+            raise RuntimeError(f"{name} must be a float32 [{H},{W}] map (m1type=cv2.CV_32FC1) on {images.device}")
+    images, map_x, map_y = images.contiguous(), map_x.contiguous(), map_y.contiguous()
+    if out is None:
+        out = torch.empty_like(images)
+    elif (not isinstance(out, torch.Tensor) or out.shape != images.shape or out.dtype != images.dtype
+          or out.device != images.device or not out.is_contiguous()):
+        raise RuntimeError("out must be a contiguous tensor of the images' shape, dtype and device")
+    if out.data_ptr() == images.data_ptr():
+        raise RuntimeError("out must not be images: the remap gathers, it cannot run in place")
+    planes = images.numel() // max(1, H * W)
+    if planes == 0:
+        return out
+    stream = torch.cuda.current_stream(images.device).cuda_stream
+    with torch.cuda.device(images.device):
+        _check(N.lib().sd_rectify(map_x.data_ptr(), map_y.data_ptr(), images.data_ptr(), out.data_ptr(),
+                                  N.SD_U8 if images.dtype == torch.uint8 else N.SD_F32, planes, H, W, stream),
+               "sd_rectify")
     return out

@@ -126,7 +126,7 @@ struct sd_handle {
     MappedWord stats;      // (its device alias is Scratch::screen_host_word)
     unsigned long long stats_seen = 0;
     int screen_pause = 0;
-    DeviceAllocs allocs;   // owns every device buffer of `s`, rmap and lr_rows
+    DeviceAllocs allocs;   // owns every device buffer of `s`, rmap, lr_rows, rect_maps and rect_frames
     Scratch s = {};
     float *dbg_cost = nullptr, *dbg_agg = nullptr;
     GrayView gv = {};      // band mode: where the left gray of the global image lives, else all zero
@@ -161,6 +161,9 @@ struct sd_handle {
     float *rmap = nullptr;       // [chunk/2][H][W] right views' disparity maps of the last chunk, in mirrored orientation
     bool lr_fill = false;        // background fill of the rejected pixels (sd_set_lr_fill)
     unsigned char *lr_rows = nullptr;   // [chunk/2][H] per row: 1 if the check kept a pixel of it (the fill's column pass)
+    // rectification (sd_set_rectification): both NULL while it is off
+    float *rect_maps = nullptr;  // [4][H][W] left map_x, left map_y, right map_x, right map_y
+    char *rect_frames = nullptr; // [2 views][chunk][3][H][W] rectified frames of the chunk in flight, uint8 or float32
     char err[640] = {};
     int last_cuda = 0;
 
@@ -376,7 +379,18 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
     const bool full = (k0 == 0 && k1 == 3);  // per-kernel profiling only brackets complete passes
     const int frames = h->lr ? 2 * pairs : pairs;
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
-    if (k0 <= 0 && 0 <= k1) SD_CUDA(h, launch_gray_pool(h->g, left, right, dtype, frames, h->s, st, h->lr ? pairs : 0));
+    if (k0 <= 0 && 0 <= k1) {
+        if (h->rect_maps) {   // raw input: remap the chunk's caller frames (once, also with the check) into rect_frames
+            const size_t n = (size_t)h->g.H * h->g.W, view_bytes = (size_t)h->chunk * 3 * n * (dtype == SD_U8 ? 1 : 4);
+            RectifyViews v;
+            v.view[0] = RectifyView{h->rect_maps, h->rect_maps + n, left, h->rect_frames};
+            v.view[1] = RectifyView{h->rect_maps + 2 * n, h->rect_maps + 3 * n, right, h->rect_frames + view_bytes};
+            SD_CUDA(h, launch_rectify(v, 2, dtype, 3 * pairs, h->g.H, h->g.W, st));
+            left = v.view[0].dst;
+            right = v.view[1].dst;
+        }
+        SD_CUDA(h, launch_gray_pool(h->g, left, right, dtype, frames, h->s, st, h->lr ? pairs : 0));
+    }
     if (full && (rc = prof_mark(h, st)) != SD_OK) return rc;
     if (k0 <= 1 && 1 <= k1) {
         h->s.range_epoch = ++h->epoch;
@@ -697,6 +711,7 @@ int sd_compute_range(sd_handle *h, const void *left, const void *right, int dtyp
     if (dtype != SD_U8 && dtype != SD_F32) return fail(h, SD_ERR_SHAPE, "dtype must be SD_U8 or SD_F32");
     if (n_frames <= 0 || n_frames > h->chunk) return fail(h, SD_ERR_SHAPE, "sd_compute_range handles at most frames_per_launch frames");
     if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "sd_compute_range (row-band mode) does not support the left-right check");
+    if (h->rect_maps) return fail(h, SD_ERR_UNSUPPORTED, "sd_compute_range (row-band mode) does not support rectification");
     DeviceGuard dg(h->device);
     if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
     int rc = order_after_previous(h, (cudaStream_t)stream);
@@ -717,6 +732,7 @@ int sd_set_band(sd_handle *h, int pooled_row_offset, int global_height, const fl
         return SD_OK;
     }
     if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check (sd_set_lr_check(h, 0, ...) first)");
+    if (h->rect_maps) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support rectification (sd_set_rectification(h, NULL, ...) first)");
     if (global_height % K != 0 || h->g.H % K != 0) return fail(h, SD_ERR_UNSUPPORTED, "band mode needs heights divisible by downscale_factor");
     if (!global_left_gray) return fail(h, SD_ERR_BAD_ARG, "band mode needs the global left gray image");
     h->g.band_x_off = pooled_row_offset;
@@ -744,6 +760,7 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     if (dtype != SD_U8 && dtype != SD_F32) return fail(h, SD_ERR_SHAPE, "dtype must be SD_U8 or SD_F32");
     if (h->p2p.on) return fail(h, SD_ERR_BAD_ARG, "sd_band_p2p_init was already called on this handle");
     if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check (sd_set_lr_check(h, 0, ...) first)");
+    if (h->rect_maps) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support rectification (sd_set_rectification(h, NULL, ...) first)");
     const Geom &g = h->g;
     const int esize = dtype == SD_U8 ? 1 : 4, K = g.K;
     if ((g.W * esize) % 16 != 0 || g.W % 4 != 0) return fail(h, SD_ERR_UNSUPPORTED, "peer-memory band mode needs 16-byte image rows");
@@ -1026,13 +1043,14 @@ int sd_launches_per_call(sd_handle *h, int n_frames) {
     if (!h || n_frames <= 0) return 0;
     // gray+pool, [pad planes for the TMA-staged specialised kernels], [level screen], cost+agg+WTA, secondary, fill
     // (left-right check: chunks of chunk/2 pairs, kernels A..C over both frames of a pair, + the checked fill;
-    //  + its row and column passes with the background fill)
+    //  + its row and column passes with the background fill; + the remap with rectification)
     int total = 0;
     const int per = h->lr ? lr_pairs(h) : h->chunk;
     const int nchunks = (n_frames + per - 1) / per, base = n_frames / nchunks, extra = n_frames % nchunks;
     for (int c = 0; c < nchunks; c++) {   // the same split as sd_compute
         const int nf = (base + (c < extra ? 1 : 0)) * (h->lr ? 2 : 1);
         total += h->lr ? (h->lr_fill ? 3 : 1) : 0;
+        total += h->rect_maps ? 1 : 0;
         const bool scr = active_variant(h, nf) == 2 && screen_active(h, nf);
         // (+2 behind the screen in reference-compat mode: absolute-index targets + gather pass)
         total += 4 + (active_variant(h, nf) >= 2 ? 1 : 0) + (scr ? 1 : 0) + (scr && h->s.agg_vol ? 2 : 0) +
@@ -1097,6 +1115,50 @@ int sd_lr_fill(const float *left_map, const float *right_map, int n, int H, int 
                                                     rows, st);
     if (cudaFreeAsync(rows, st) != cudaSuccess || e != cudaSuccess) return SD_ERR_CUDA;
     return SD_OK;
+}
+
+int sd_set_rectification(sd_handle *h, const float *left_map_x, const float *left_map_y, const float *right_map_x,
+                         const float *right_map_y, void *cuda_stream) {
+    if (!h) return SD_ERR_BAD_ARG;
+    const int given = !!left_map_x + !!left_map_y + !!right_map_x + !!right_map_y;
+    if (given != 0 && given != 4) return fail(h, SD_ERR_BAD_ARG, "pass all four maps, or all four NULL to switch rectification off");
+    DeviceGuard dg(h->device);
+    if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
+    if (given == 0) {   // (cudaFree waits for the chunks still reading the buffers)
+        h->allocs.release(h->rect_maps);
+        h->allocs.release(h->rect_frames);
+        return SD_OK;
+    }
+    if (h->gv.flat || h->p2p.on) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support rectification");
+    if (h->g.H >= 32768 || h->g.W >= 32768) return fail(h, SD_ERR_UNSUPPORTED, "rectification needs H, W < 32768 (as cv2.remap)");
+    const size_t n = (size_t)h->g.H * h->g.W;
+    if (!h->rect_maps) {
+        SD_CUDA(h, h->allocs.alloc(&h->rect_maps, 4 * n * sizeof(float)));
+        const cudaError_t e = h->allocs.alloc(&h->rect_frames, (size_t)h->chunk * 2 * 3 * n * sizeof(float));
+        if (e != cudaSuccess) {
+            h->allocs.release(h->rect_maps);
+            return fail_cuda(h, e, "sd_set_rectification (rectified frames)");
+        }
+    }
+    // the previous call's chunks may still read the old maps: the copies follow them on cuda_stream
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    int rc = order_after_previous(h, st);
+    if (rc != SD_OK) return rc;
+    const float *src[4] = {left_map_x, left_map_y, right_map_x, right_map_y};
+    for (int i = 0; i < 4; i++)
+        SD_CUDA(h, cudaMemcpyAsync(h->rect_maps + i * n, src[i], n * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    return mark_last_use(h, st);
+}
+
+int sd_rectify(const float *map_x, const float *map_y, const void *src, void *dst, int dtype, int n_planes, int H, int W,
+               void *cuda_stream) {
+    if (!map_x || !map_y || !src || !dst || n_planes <= 0 || H <= 0 || W <= 0) return SD_ERR_BAD_ARG;
+    if (dtype != SD_U8 && dtype != SD_F32) return SD_ERR_BAD_ARG;
+    if (H >= 32768 || W >= 32768) return SD_ERR_BAD_ARG;
+    if (dst == src) return SD_ERR_BAD_ARG;   // a gather cannot run in place
+    RectifyViews v = {};
+    v.view[0] = RectifyView{map_x, map_y, src, dst};
+    return launch_rectify(v, 1, dtype, n_planes, H, W, (cudaStream_t)cuda_stream) == cudaSuccess ? SD_OK : SD_ERR_CUDA;
 }
 
 int sd_set_level_split(sd_handle *h, int on) {

@@ -166,6 +166,18 @@ cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const Gr
 cudaError_t launch_lr_background_fill(const float *left, const float *right, bool right_mirrored, int frames, int H, int W,
                                       float tolerance, float invalid, float *out, unsigned char *row_kept,
                                       cudaStream_t st);
+// Rectification remap (rectify.cu, DESIGN.md §14), exactly cv2.remap with CV_32FC1 maps, INTER_LINEAR and a constant 0
+// border: dst[p][r][c] = src[p] sampled at (map_x[r][c], map_y[r][c]) for `planes` [H][W] planes per view, uint8 or
+// float32 by `dtype`; grid.y runs over the n_views (1 or 2) views.  H, W < 32768; dst must not overlap src.
+struct RectifyView {
+    const float *map_x, *map_y;
+    const void *src;
+    void *dst;
+};
+struct RectifyViews {
+    RectifyView view[2];
+};
+cudaError_t launch_rectify(const RectifyViews &v, int n_views, int dtype, int planes, int H, int W, cudaStream_t st);
 // peer-memory row-band exchange (band_p2p.cu)
 cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l, void *own_r, void *prev_l, void *prev_r,
                                 void *next_l, void *next_r, int row_bytes, int band_rows, int halo, int own_rows, int prev_rows,

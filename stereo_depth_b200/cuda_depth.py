@@ -12,7 +12,8 @@ Differences from the reference, all additive:
   * kernels run on PyTorch's current stream (the reference uses the legacy default stream);
   * `compute_disparity_batch` processes [N,3,H,W] in one call;
   * `set_left_right_check` marks occluded and mismatched pixels with an invalid value, or fills them from the
-    background (off by default).
+    background (off by default);
+  * `set_rectification` takes raw frames from an unrectified rig and remaps them on the GPU first (off by default).
 """
 import math
 
@@ -70,6 +71,7 @@ class StereoMatching:
         self._out = torch.empty((self.height, self.width), dtype=torch.float32, device=self._dev())
         self._lr_tolerance = None
         self._lr_fill = False
+        self._rectification = False
 
     def _dev(self):
         return torch.device("cuda", self._device)
@@ -181,6 +183,46 @@ class StereoMatching:
     def background_fill(self):
         """True while the left-right check fills the pixels it rejects instead of marking them invalid."""
         return self._lr_fill
+
+    def _map_tensor(self, m, name):
+        if isinstance(m, torch.Tensor):
+            t = m
+        else:
+            import numpy as np
+            if not isinstance(m, np.ndarray):
+                raise TypeError(f"{name} must be a numpy array or a torch tensor, got {type(m).__name__}")
+            t = torch.from_numpy(m)
+        if t.dtype != torch.float32 or tuple(t.shape) != (self.height, self.width):
+            raise RuntimeError(f"{name} must be a float32 [{self.height},{self.width}] map (cv2.initUndistortRectifyMap "
+                               f"with m1type=cv2.CV_32FC1), got {t.dtype} {list(t.shape)}")
+        return t.to(self._dev()).contiguous()
+
+    def set_rectification(self, left_maps, right_maps):
+        """Rectify raw frames on the GPU before matching, on every entry point of this matcher (default off).
+
+        left_maps / right_maps: (map_x, map_y) of each view as cv2.initUndistortRectifyMap returns them with
+        m1type=cv2.CV_32FC1 -- float32 [H,W] numpy arrays or tensors giving, for every rectified pixel, the raw image's
+        sampling coordinate.  Every view is then remapped exactly as cv2.remap(raw, map_x, map_y, cv2.INTER_LINEAR,
+        borderMode=cv2.BORDER_CONSTANT, borderValue=0) would (DESIGN.md §14), and the outputs are in rectified (left)
+        coordinates.  The maps are copied to the matcher's device, so the caller may change theirs afterwards.
+        `set_rectification(None, None)` switches it off."""
+        if left_maps is None and right_maps is None:
+            self._handle.set_rectification(None, None, None, None, None)
+            self._rectification = False
+            return
+        maps = []
+        for pair, view in ((left_maps, "left"), (right_maps, "right")):
+            if pair is None or len(pair) != 2:
+                raise RuntimeError(f"{view}_maps must be a (map_x, map_y) pair, or both maps None to switch off")
+            maps += [self._map_tensor(m, f"{view} map_{a}") for m, a in zip(pair, "xy")]
+        stream = torch.cuda.current_stream(self._dev()).cuda_stream
+        self._handle.set_rectification(*[m.data_ptr() for m in maps], stream)
+        self._rectification = True
+
+    @property
+    def rectification(self):
+        """True while this matcher rectifies its input frames (set_rectification)."""
+        return self._rectification
 
     # ---- parity / debugging hooks (not part of the reference API) -------------------------------
     def stage(self, name, frame=0):

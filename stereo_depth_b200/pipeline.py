@@ -54,6 +54,9 @@ class DepthEstimationPipelineConfig:
     left_right_check: Optional[float] = None
     # with left_right_check: fill the pixels it rejects from the background (DESIGN.md §13) instead of marking them
     left_right_background_fill: bool = False
+    # raw (unrectified) frames: ((left map_x, left map_y), (right map_x, right map_y)) from cv2.initUndistortRectifyMap
+    # with m1type=cv2.CV_32FC1; every frame is rectified on the GPU before matching (None = frames are rectified)
+    rectification_maps: Optional[Tuple[Any, Any]] = None
 
     def update(self, **kwargs: Any) -> "DepthEstimationPipelineConfig":
         for key, value in kwargs.items():
@@ -113,6 +116,8 @@ class DepthEstimationPipeline:
                 max_disparity=self._config.max_disparity,
             )
             backend = CudaStereoMatchingBackend(configuration=config)
+            if self._config.rectification_maps is not None:
+                backend.native.set_rectification(*self._config.rectification_maps)
             if self._config.left_right_check is not None:
                 backend.native.set_left_right_check(self._config.left_right_check, self._config.invalid_disparity,
                                                     self._config.left_right_background_fill)

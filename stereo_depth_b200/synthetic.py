@@ -75,6 +75,64 @@ def make_layered_pair(H, W, D, seed=1234):
     return left, right, gt.astype(np.float32), visible
 
 
+def _bilinear(img, x, y):
+    """float32 [C,H,W] image sampled at float coordinates x, y ([H',W']); zero outside."""
+    C, H, W = img.shape
+    x0, y0 = np.floor(x).astype(np.int64), np.floor(y).astype(np.int64)
+    ax, ay = (x - x0).astype(np.float32), (y - y0).astype(np.float32)
+    out = np.zeros((C,) + x.shape, np.float32)
+    for dy, dx, w in ((0, 0, (1 - ay) * (1 - ax)), (0, 1, (1 - ay) * ax), (1, 0, ay * (1 - ax)), (1, 1, ay * ax)):
+        yy, xx = y0 + dy, x0 + dx
+        inside = (yy >= 0) & (yy < H) & (xx >= 0) & (xx < W)
+        out += np.where(inside, img[:, np.clip(yy, 0, H - 1), np.clip(xx, 0, W - 1)], 0) * w
+    return out
+
+
+def _rotation(pitch, roll):
+    cp, sp, cr, sr = np.cos(pitch), np.sin(pitch), np.cos(roll), np.sin(roll)
+    about_x = np.array([[1, 0, 0], [0, cp, -sp], [0, sp, cp]])
+    about_z = np.array([[cr, -sr, 0], [sr, cr, 0], [0, 0, 1]])
+    return about_z @ about_x
+
+
+def make_unrectified_pair(H, W, D, seed=1234, degrees=1.0):
+    """A make_pair scene as a stereo rig whose cameras are slightly rotated about their optical centres: the left camera
+    by +degrees of pitch and +degrees/2 of roll, the right one by the opposite.  Focal length W pixels, principal point
+    at the image centre.  A rotation about the optical centre maps the rectified image by the homography
+    Hm = Kc R Kc^-1 (rectified pixel -> raw pixel), so the raw views are the rectified ones resampled (bilinear, zero
+    outside) at Hm^-1, and the rectification maps are Hm itself -- what cv2.initUndistortRectifyMap gives for such a rig
+    without lens distortion.  Returns (left_raw u8 [3,H,W], right_raw u8 [3,H,W],
+    ((left map_x, left map_y), (right map_x, right map_y)) float32 [H,W] each, gt int32 [H,W] in rectified left
+    coordinates)."""
+    left, right, gt = make_pair(H, W, D, seed)
+    raws = []
+    for img, (Hm, pix) in zip((left, right), _rotated_rig(H, W, degrees)):
+        q = np.einsum("ij,jhw->ihw", np.linalg.inv(Hm), pix)
+        raw = _bilinear(img.astype(np.float32), q[0] / q[2], q[1] / q[2])
+        raws.append(np.clip(np.rint(raw), 0, 255).astype(np.uint8))
+    return raws[0], raws[1], rotated_rig_maps(H, W, degrees), gt
+
+
+def _rotated_rig(H, W, degrees):
+    """(homography rectified -> raw pixel, homogeneous pixel grid [3,H,W]) of the left and the right camera."""
+    f = float(W)
+    Kc = np.array([[f, 0, (W - 1) / 2], [0, f, (H - 1) / 2], [0, 0, 1]])
+    a = np.deg2rad(degrees)
+    cols, rows = np.meshgrid(np.arange(W, dtype=np.float64), np.arange(H, dtype=np.float64))
+    pix = np.stack([cols, rows, np.ones_like(cols)])
+    return [(Kc @ _rotation(s * a, s * a / 2) @ np.linalg.inv(Kc), pix) for s in (1.0, -1.0)]
+
+
+def rotated_rig_maps(H, W, degrees=1.0):
+    """The rectification maps of make_unrectified_pair's rig without rendering its views:
+    ((left map_x, left map_y), (right map_x, right map_y)), float32 [H,W] each."""
+    out = []
+    for Hm, pix in _rotated_rig(H, W, degrees):
+        p = np.einsum("ij,jhw->ihw", Hm, pix)
+        out.append(((p[0] / p[2]).astype(np.float32), (p[1] / p[2]).astype(np.float32)))
+    return out[0], out[1]
+
+
 def make_batch(n, H, W, D, seed=1234, first_frame=0):
     ls, rs = [], []
     for f in range(n):
