@@ -237,6 +237,18 @@ int sd_set_rectification(sd_handle *h, const float *left_map_x, const float *lef
 int sd_rectify(const float *map_x, const float *map_y, const void *src, void *dst, int dtype, int n_planes, int H, int W,
                void *cuda_stream);
 
+/* Reprojection of disparity maps to metric 3-D points, exactly cv2.reprojectImageTo3D(disparity, Q, xyz,
+ * handleMissingValues) with float32 maps (rule: DESIGN.md §15): n float32 [H][W] maps at `disparity` (device memory)
+ * -> xyz = n float32 [H][W][3] point maps (X, Y, Z interleaved, OpenCV's CV_32FC3; device memory).  Q: the 4x4
+ * reprojection matrix of cv2.stereoRectify as 16 row-major doubles in HOST memory, read during the call.  With
+ * handle_missing_values != 0 every pixel whose disparity lies within FLT_EPSILON of its frame's minimum gets Z = 10000;
+ * the minimum is taken over the non-NaN values (OpenCV's is undefined with NaN) and a frame that is all NaN has none.
+ * Asynchronous on cuda_stream (handle_missing_values allocates n * 4 bytes of scratch with cudaMallocAsync and adds one
+ * launch).  SD_ERR_BAD_ARG for null pointers, n, H or W <= 0, or xyz overlapping disparity; SD_ERR_CUDA if a launch
+ * fails. */
+int sd_reproject(const float *disparity, int n, int H, int W, const double *Q, int handle_missing_values, float *xyz,
+                 void *cuda_stream);
+
 /* Level split for launches that cannot fill the GPU (one small frame, a thin row band): the unscreened specialised
  * kernel then spreads every tile's disparity levels over several blocks and a small kernel merges the partial
  * winner-take-all records (identical results: the maximum is taken in ascending level order with strict '>').

@@ -20,7 +20,7 @@ CONFIG_FIELDS = ("height", "width", "downscale_factor", "min_disparity", "max_di
 EXPORTS = ("sd_abi_version", "sd_config_default", "sd_dims", "sd_create", "sd_destroy", "sd_compute",
            "sd_compute_range", "sd_set_band", "sd_band_p2p_init", "sd_band_p2p_connect", "sd_band_p2p_compute", "sd_compute_host", "sd_get_stage", "sd_set_debug_volumes", "sd_set_compat", "sd_set_variant",
            "sd_launches_per_call", "sd_frames_per_launch", "sd_active_variant", "sd_set_screen", "sd_screen_active", "sd_screen_stats", "sd_screen_paused", "sd_profile_enable", "sd_profile_read", "sd_profile_read_detail", "sd_metrics", "sd_point_cloud", "sd_check_guards", "sd_stage_pointer", "sd_set_debug_screen", "sd_set_level_split", "sd_level_split",
-           "sd_set_lr_check", "sd_set_lr_fill", "sd_lr_fill", "sd_set_rectification", "sd_rectify", "sd_last_error", "sd_last_cuda_error")
+           "sd_set_lr_check", "sd_set_lr_fill", "sd_lr_fill", "sd_set_rectification", "sd_rectify", "sd_reproject", "sd_last_error", "sd_last_cuda_error")
 
 
 class SdConfig(C.Structure):
@@ -86,6 +86,7 @@ def lib():
     L.sd_lr_fill.argtypes = [vp, vp, ip, ip, ip, C.c_float, C.c_float, vp, vp]
     L.sd_set_rectification.argtypes = [vp, vp, vp, vp, vp, vp]
     L.sd_rectify.argtypes = [vp, vp, vp, vp, ip, ip, ip, ip, vp]
+    L.sd_reproject.argtypes = [vp, ip, ip, ip, C.POINTER(C.c_double), ip, vp, vp]
     L.sd_check_guards.argtypes = [vp, C.POINTER(C.c_longlong)]
     L.sd_last_error.argtypes = [vp]
     L.sd_last_error.restype = C.c_char_p

@@ -2,9 +2,12 @@
 accuracy metrics (depth_estimation_pipeline_metrics.py:18-56) and the point cloud
 (depth_estimation_pipeline_hooks.py:84-92, helpers/point_cloud_helpers.py:5-13); and the left-right check with the
 background fill for callers that hold both views' disparity maps; and the rectification remap for callers that want
-a rectified image itself (to colour a point cloud or display a map)."""
+a rectified image itself (to colour a point cloud or display a map); and cv2.reprojectImageTo3D, the metric point
+map of a calibrated rig."""
+import ctypes
 import math
 
+import numpy as np
 import torch
 
 from . import _native as N
@@ -111,4 +114,48 @@ def rectify(images: torch.Tensor, map_x: torch.Tensor, map_y: torch.Tensor, out=
         _check(N.lib().sd_rectify(map_x.data_ptr(), map_y.data_ptr(), images.data_ptr(), out.data_ptr(),
                                   N.SD_U8 if images.dtype == torch.uint8 else N.SD_F32, planes, H, W, stream),
                "sd_rectify")
+    return out
+
+
+def reprojection_matrix(Q) -> np.ndarray:
+    """Q (cv2.stereoRectify's 4x4 reprojection matrix: numpy array, tensor or nested lists of any integer or float
+    dtype) as a contiguous float64 numpy array, the conversion cv2.reprojectImageTo3D makes (it refuses bool)."""
+    if isinstance(Q, torch.Tensor):
+        Q = Q.detach().cpu().numpy()
+    q = np.asarray(Q)
+    if q.shape != (4, 4) or q.dtype.kind not in "iuf":
+        raise RuntimeError(f"Q must be a 4x4 integer or floating-point matrix (cv2.stereoRectify's Q), got {q.dtype} "
+                           f"{q.shape}")
+    return np.ascontiguousarray(q, dtype=np.float64)
+
+
+def reproject_image_to_3d(disparity: torch.Tensor, Q, handle_missing_values: bool = False, out=None):
+    """cv2.reprojectImageTo3D(disparity, Q, handleMissingValues=handle_missing_values) of a [H,W] or [N,H,W] float32
+    CUDA disparity map, bit for bit (DESIGN.md §15): [..., H, W, 3] float32 points (X, Y, Z).  Q: 4x4 of any integer or
+    float dtype, converted to float64 as OpenCV does.  With handle_missing_values, pixels within FLT_EPSILON of their
+    frame's minimum disparity get Z = 10000; the minimum is over the non-NaN values (OpenCV's is undefined with NaN).
+    Returns `out` (a new tensor when None), which must not overlap `disparity`."""
+    if not isinstance(disparity, torch.Tensor):
+        raise TypeError("disparity must be a tensor")
+    if disparity.dim() not in (2, 3) or not disparity.is_cuda or disparity.dtype != torch.float32:
+        raise RuntimeError("disparity must be a float32 CUDA tensor of shape [H,W] or [N,H,W]")
+    q = reprojection_matrix(Q)
+    disparity = disparity.contiguous()
+    shape = tuple(disparity.shape) + (3,)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.float32, device=disparity.device)
+    elif (not isinstance(out, torch.Tensor) or tuple(out.shape) != shape or out.dtype != torch.float32
+          or out.device != disparity.device or not out.is_contiguous()):
+        raise RuntimeError(f"out must be a contiguous float32 tensor of shape {list(shape)} on {disparity.device}")
+    if disparity.numel() == 0:
+        return out
+    d0, x0 = disparity.data_ptr(), out.data_ptr()
+    if x0 < d0 + 4 * disparity.numel() and d0 < x0 + 4 * out.numel():
+        raise RuntimeError("out must not overlap disparity")
+    n = 1 if disparity.dim() == 2 else disparity.shape[0]
+    H, W = disparity.shape[-2:]
+    stream = torch.cuda.current_stream(disparity.device).cuda_stream
+    with torch.cuda.device(disparity.device):
+        _check(N.lib().sd_reproject(d0, n, H, W, q.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                                    1 if handle_missing_values else 0, x0, stream), "sd_reproject")
     return out

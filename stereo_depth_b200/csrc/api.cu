@@ -1161,6 +1161,25 @@ int sd_rectify(const float *map_x, const float *map_y, const void *src, void *ds
     return launch_rectify(v, 1, dtype, n_planes, H, W, (cudaStream_t)cuda_stream) == cudaSuccess ? SD_OK : SD_ERR_CUDA;
 }
 
+int sd_reproject(const float *disparity, int n, int H, int W, const double *Q, int handle_missing_values, float *xyz,
+                 void *cuda_stream) {
+    if (!disparity || !Q || !xyz || n <= 0 || H <= 0 || W <= 0) return SD_ERR_BAD_ARG;
+    const unsigned long long hw = (unsigned long long)H * W;
+    if ((unsigned long long)n > (1ull << 58) / hw) return SD_ERR_BAD_ARG;   // larger than any buffer: 12 * px must not wrap
+    const unsigned long long px = n * hw;
+    const uintptr_t d0 = (uintptr_t)disparity, d1 = d0 + 4 * px, x0 = (uintptr_t)xyz, x1 = x0 + 12 * px;
+    if (x0 < d1 && d0 < x1) return SD_ERR_BAD_ARG;                 // the points would overwrite maps still to be read
+    ReprojectQ q;
+    memcpy(q.q, Q, sizeof(q.q));
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    unsigned *mins = nullptr;
+    if (handle_missing_values && cudaMallocAsync((void **)&mins, (size_t)n * sizeof(unsigned), st) != cudaSuccess)
+        return SD_ERR_CUDA;
+    const cudaError_t e = launch_reproject(disparity, n, H, W, q, mins, xyz, st);
+    if ((mins && cudaFreeAsync(mins, st) != cudaSuccess) || e != cudaSuccess) return SD_ERR_CUDA;
+    return SD_OK;
+}
+
 int sd_set_level_split(sd_handle *h, int on) {
     if (!h) return SD_ERR_BAD_ARG;
     h->split_off = (on == 0);

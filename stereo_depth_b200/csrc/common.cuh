@@ -178,6 +178,14 @@ struct RectifyViews {
     RectifyView view[2];
 };
 cudaError_t launch_rectify(const RectifyViews &v, int n_views, int dtype, int planes, int H, int W, cudaStream_t st);
+// Reprojection to 3-D (reproject.cu, DESIGN.md §15), exactly cv2.reprojectImageTo3D: n float32 [H][W] disparity maps ->
+// xyz [n][H][W][3] float32 with the 4x4 row-major Q.  min_key: n unsigned of scratch for handleMissingValues (one more
+// launch plus a memset), NULL without it.  xyz must not overlap disp.
+struct ReprojectQ {
+    double q[16];
+};
+cudaError_t launch_reproject(const float *disp, int n, int H, int W, const ReprojectQ &Q, unsigned *min_key, float *xyz,
+                             cudaStream_t st);
 // peer-memory row-band exchange (band_p2p.cu)
 cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l, void *own_r, void *prev_l, void *prev_r,
                                 void *next_l, void *next_r, int row_bytes, int band_rows, int halo, int own_rows, int prev_rows,

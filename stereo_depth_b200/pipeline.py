@@ -25,7 +25,7 @@ from typing import Any, Dict, Iterable, Iterator, List, Optional, Tuple
 
 import torch
 
-from . import cuda_depth
+from . import consumers, cuda_depth
 from .backend import CudaStereoMatchingBackend, StereoMatching
 
 
@@ -57,6 +57,9 @@ class DepthEstimationPipelineConfig:
     # raw (unrectified) frames: ((left map_x, left map_y), (right map_x, right map_y)) from cv2.initUndistortRectifyMap
     # with m1type=cv2.CV_32FC1; every frame is rectified on the GPU before matching (None = frames are rectified)
     rectification_maps: Optional[Tuple[Any, Any]] = None
+    # the 4x4 reprojection matrix Q of cv2.stereoRectify, in the coordinates of the disparity map (the rectified left
+    # view with rectification_maps): every result then carries its metric points (consumers.reproject_image_to_3d)
+    reprojection_matrix: Optional[Any] = None
 
     def update(self, **kwargs: Any) -> "DepthEstimationPipelineConfig":
         for key, value in kwargs.items():
@@ -71,6 +74,7 @@ class DepthEstimationResult:
     left_image: torch.Tensor
     right_image: torch.Tensor
     disparity_map: torch.Tensor
+    points: Optional[torch.Tensor] = None   # [H,W,3] float32 (X, Y, Z) when config.reprojection_matrix is set
 
 
 @dataclass
@@ -80,6 +84,7 @@ class DepthEstimationPipelineContext:
     right_image: torch.Tensor
     config: DepthEstimationPipelineConfig
     frame_index: int
+    points: Optional[torch.Tensor] = None
 
 
 class DepthEstimationPipeline:
@@ -87,6 +92,8 @@ class DepthEstimationPipeline:
     def __init__(self, config: Optional[DepthEstimationPipelineConfig] = None, right_view_synthesis=None):
         self._config = config if config is not None else DepthEstimationPipelineConfig()
         self._right_view_synthesis = right_view_synthesis
+        self._reprojection = (None if self._config.reprojection_matrix is None
+                              else consumers.reprojection_matrix(self._config.reprojection_matrix))
         self._stereo_matching = self._get_stereo_matching()
 
     def process(self, left_image: torch.Tensor, right_image: Optional[torch.Tensor] = None) -> DepthEstimationResult:
@@ -99,7 +106,12 @@ class DepthEstimationPipeline:
                 right_image = self._right_view_synthesis.process(left_image)
         with cuda_perf_clock("Stereo matching", self._config.log_perf_time):
             disparity_map = self._stereo_matching.process(left_image, right_image)
-        return DepthEstimationResult(disparity_map=disparity_map, left_image=left_image, right_image=right_image)
+        points = None
+        if self._reprojection is not None:
+            with cuda_perf_clock("Reprojection", self._config.log_perf_time):
+                points = consumers.reproject_image_to_3d(disparity_map, self._reprojection)
+        return DepthEstimationResult(disparity_map=disparity_map, left_image=left_image, right_image=right_image,
+                                     points=points)
 
     def get_configuration(self) -> DepthEstimationPipelineConfig:
         return self._config
@@ -199,7 +211,8 @@ def run_depth_estimation_pipeline(camera, pipeline: DepthEstimationPipeline, hoo
         _check_frame_shape(config, left_view)
         result = pipeline.process(left_view, right_view)
         context = DepthEstimationPipelineContext(disparity_map=result.disparity_map, left_image=result.left_image,
-                                                 right_image=result.right_image, config=config, frame_index=frame_index)
+                                                 right_image=result.right_image, config=config, frame_index=frame_index,
+                                                 points=result.points)
         for hook in hooks:
             hook.process(context)
     for hook in hooks:
@@ -260,7 +273,6 @@ def run_depth_estimation_pipeline_evaluation(camera, pipeline: DepthEstimationPi
     (`stream_image_pairs_with_gt_disparity`, camera/camera.py:30-35) or is a plain iterable of (left, right, gt_disparity).
     D1 / Threshold_n / MAE come from ONE fused pass per frame (consumers.evaluate, mask 0 < gt <= max_disparity); any other metric object is called
     with the reference's (estimate, gt, mask) arguments."""
-    from . import consumers
     metrics = list(metrics or [])
     results: Dict[str, List[float]] = {m.name(): [] for m in metrics}
     config = pipeline.get_configuration()
