@@ -461,12 +461,9 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
 }
 
 // Frames per chunk of the pipelined host path: copies of a chunk cannot overlap its own kernels, so the host path uses
-// chunks of at most 8 frames whatever the device path's chunk is (SD_HOST_CHUNK: tuning knob).
-int host_chunk(const sd_handle *h) {
-    static const int env_hc = getenv("SD_HOST_CHUNK") ? atoi(getenv("SD_HOST_CHUNK")) : 0;
-    const int want = env_hc > 0 ? env_hc : 8;
-    return h->chunk < want ? h->chunk : want;
-}
+// chunks of at most kHostChunk frames whatever the device path's chunk is.
+constexpr int kHostChunk = 8;
+int host_chunk(const sd_handle *h) { return h->chunk < kHostChunk ? h->chunk : kHostChunk; }
 
 // frames (pairs with the left-right check) per host-path chunk: the slots hold host_chunk frames, scratch 2 * pairs
 int host_chunk_frames(const sd_handle *h) {
@@ -900,11 +897,10 @@ int sd_compute_host(sd_handle *h, const void *left, const void *right, int dtype
     const size_t inb = in_bytes_per_frame(h, dtype), outn = (size_t)h->g.H * h->g.W;
     // Chunk schedule: a short first chunk (its H2D copy cannot overlap anything) and a short last chunk (neither
     // can its D2H copy); full chunks in between keep the fused kernel's wave quantisation efficient.
-    // Copies of a chunk cannot overlap its own kernels, so the host path uses chunks of at most 8 frames (the
+    // Copies of a chunk cannot overlap its own kernels, so the host path uses chunks of at most kHostChunk frames (the
     // device path's larger default only matters for the fused kernel's wave quantisation).
-    static const int env_edge = getenv("SD_HOST_EDGE") ? atoi(getenv("SD_HOST_EDGE")) : 0;   // tuning knob
     const int hc = host_chunk_frames(h);
-    const int edge = (hc >= 4 && n_frames >= 3 * hc) ? (env_edge > 0 ? env_edge : 2) : hc;
+    const int edge = (hc >= 4 && n_frames >= 3 * hc) ? 2 : hc;
     int it = 0;
     // On any failure below, copies to / from the caller's host buffers may still be in flight: drain before returning.
     struct Drain {

@@ -16,14 +16,12 @@
 //     and reused by all L/2 passes;
 //   * the 3x3 cost is computed by row-streaming 4-column strips: every |L-R| tap is evaluated once and
 //     reused by the 3 cost rows and up to 3 cost columns that contain it;
-//   * WTA keeps only (best, previous level) in registers and rewrites a pixel's 16-byte record
-//     (d*, A[d*-1], A[d*], A[d*+1]) when its maximum improves; the [Hd,Wd,L] volume never exists.
+//   * WTA keeps only (best, previous level, one pending A[d-1]) in registers and writes a pixel's 16-byte record
+//     (d*, A[d*-1], A[d*], A[d*+1]) once it is complete and still standing; the [Hd,Wd,L] volume never exists.
 //
 // Semantics: identical to mbm_wta_generic.cu / oracle so_cost + so_aggregate + so_wta (SAFE padding).
 // References: device_functions.cuh:53-73, ncc_matching_cost_volume_construction.cu:67-76,
 // multi_block_matching_cost_aggregation.cu:56-87, wta_disparity_selection.cu:22-30.
-#include <stdlib.h>
-
 #include <type_traits>
 
 #include "common.cuh"
@@ -54,7 +52,7 @@ __host__ __device__ inline size_t smem_bytes(int L, int min_ds) {
 // STORE: 0 nothing, 1 the whole aggregated volume (plane-major), 2 GATHER: no WTA at all, the flagged pairs' values go
 // to the compact per-tile volume (Geom::abs_index == 2) and wta4 / edge2 are left untouched.
 // SPLIT: level split (n_split_arg > 1 parts per tile); false compiles the part logic away (n_split == 1).
-template <int BH, bool DBG, int MODE, int STORE, bool SPLIT>
+template <int BH, bool DBG, int STORE, bool SPLIT>
 __global__ void __launch_bounds__(Cfg<BH>::NT, (BH <= 32) ? 2 : 1)
 mbm_wta_fast_kernel(Geom g, PadGeom pg, const float *__restrict__ padl, const float *__restrict__ padr,
                     float4 *__restrict__ wta4, float2 *__restrict__ edge2, float *__restrict__ dbg_cost,
@@ -146,10 +144,10 @@ mbm_wta_fast_kernel(Geom g, PadGeom pg, const float *__restrict__ padl, const fl
     }
 
     // ---- per-pixel WTA state (16 pixels, index k = a*4 + b) ---------------------------------------
-    // Only the running maximum and the previous level stay in registers.  Whenever a pixel's maximum
-    // improves, its record (d*, A[d*-1], A[d*], A[d*+1]) is (re)written to HBM/L2 -- about ln(L) times per
-    // pixel -- which keeps ~50 registers free for the adder chains.  Pixels outside the image start at
-    // +inf and therefore never store.
+    // Only the running maximum, the previous level and one pending A[d-1] stay in registers.  A pixel's record
+    // (d*, A[d*-1], A[d*], A[d*+1]) goes to HBM/L2 once it is complete and still standing (see the WTA update
+    // below) -- at most about ln(L) times per pixel -- which keeps ~50 registers free for the adder chains.
+    // Pixels outside the image start at +inf and therefore never store.
     float best[16], prev[16], pam[16];
     unsigned pend = 0;  // bit k: pixel k's maximum sits at the odd level of the last evaluated pair; its record (with
                         // pam[k] = A[d*-1]) is written when the next pair delivers A[d*+1], or at the end
@@ -320,35 +318,27 @@ mbm_wta_fast_kernel(Geom g, PadGeom pg, const float *__restrict__ padl, const fl
             vrow(vp + 1 * NCHUNK, 0, 1, 1);
             vrow(vp + 2 * NCHUNK, 0, 2, 2);
             vrow(vp + 3 * NCHUNK, 0, 3, 3);
-            if ((MODE & 3) == 1) {
+            // rows 4 .. 20, where every pixel row's window is open: a manual software pipeline issues the next row's
+            // loads before this row's adds (measured faster than the rolled and the fully unrolled loop, DESIGN.md §4-B)
+            auto vload = [&](const float4 *p, float4(&q)[4]) { q[0] = p[0]; q[1] = p[HALF]; q[2] = p[1]; q[3] = p[HALF + 1]; };
+            auto vcomp = [&](const float4(&q)[4]) {
+                const float2 w[8] = {lo2(q[0]), hi2(q[0]), lo2(q[1]), hi2(q[1]), lo2(q[2]), hi2(q[2]), lo2(q[3]), hi2(q[3])};
 #pragma unroll
-                for (int t = 4; t <= 20; t++) vrow(vp + t * NCHUNK, 0, 3, -1);
-            } else if ((MODE & 3) == 2) {
-                // manual software pipeline: the next row's loads are issued before this row's adds
-                auto vload = [&](const float4 *p, float4(&q)[4]) { q[0] = p[0]; q[1] = p[HALF]; q[2] = p[1]; q[3] = p[HALF + 1]; };
-                auto vcomp = [&](const float4(&q)[4]) {
-                    const float2 w[8] = {lo2(q[0]), hi2(q[0]), lo2(q[1]), hi2(q[1]), lo2(q[2]), hi2(q[2]), lo2(q[3]), hi2(q[3])};
+                for (int c3 = 0; c3 < 3; c3++)
 #pragma unroll
-                    for (int c3 = 0; c3 < 3; c3++)
-#pragma unroll
-                        for (int k = 0; k < 16; k++) acc[k] = __fadd2_rn(acc[k], w[(k & 3) + 1 + c3]);
-                };
-                float4 qa[4], qb[4];
-                const float4 *p = vp + 4 * NCHUNK;
-                vload(p, qa);
+                    for (int k = 0; k < 16; k++) acc[k] = __fadd2_rn(acc[k], w[(k & 3) + 1 + c3]);
+            };
+            float4 qa[4], qb[4];
+            const float4 *p = vp + 4 * NCHUNK;
+            vload(p, qa);
 #pragma unroll 1
-                for (int t = 4; t < 20; t += 2, p += 2 * NCHUNK) {
-                    vload(p + NCHUNK, qb);
-                    vcomp(qa);
-                    vload(p + 2 * NCHUNK, qa);
-                    vcomp(qb);
-                }
-                vcomp(qa);  // row 20
-            } else {
-                const float4 *p = vp + 4 * NCHUNK;
-#pragma unroll 2
-                for (int t = 4; t <= 20; t++, p += NCHUNK) vrow(p, 0, 3, -1);
+            for (int t = 4; t < 20; t += 2, p += 2 * NCHUNK) {
+                vload(p + NCHUNK, qb);
+                vcomp(qa);
+                vload(p + 2 * NCHUNK, qa);
+                vcomp(qb);
             }
+            vcomp(qa);  // row 20
             vrow(vp + 21 * NCHUNK, 1, 3, -1);
             vrow(vp + 22 * NCHUNK, 2, 3, -1);
             vrow(vp + 23 * NCHUNK, 3, 3, -1);
@@ -381,14 +371,9 @@ mbm_wta_fast_kernel(Geom g, PadGeom pg, const float *__restrict__ padl, const fl
             crow(cp + 1 * NCHUNK, 0, 1, 1);
             crow(cp + 2 * NCHUNK, 0, 2, 2);
             crow(cp + 3 * NCHUNK, 0, 3, 3);
-            if (MODE & 4) {
-#pragma unroll
-                for (int t = 4; t <= 8; t++) crow(cp + t * NCHUNK, 0, 3, -1);
-            } else {
-                const float4 *p = cp + 4 * NCHUNK;
+            const float4 *p = cp + 4 * NCHUNK;
 #pragma unroll 1
-                for (int t = 4; t <= 8; t++, p += NCHUNK) crow(p, 0, 3, -1);
-            }
+            for (int t = 4; t <= 8; t++, p += NCHUNK) crow(p, 0, 3, -1);
             crow(cp + 9 * NCHUNK, 1, 3, -1);
             crow(cp + 10 * NCHUNK, 2, 3, -1);
             crow(cp + 11 * NCHUNK, 3, 3, -1);
@@ -560,13 +545,13 @@ __global__ void merge_parts_kernel(const float4 *__restrict__ pw, const float2 *
     if (p_first >= 0) edge2[i] = make_float2(pe[(size_t)p_first * n + i].x, pe[(size_t)p_last * n + i].y);
 }
 
-template <int BH, bool DBG, int MODE, int STORE>
+template <int BH, bool DBG, int STORE>
 cudaError_t launch_t(const Geom &g, int frames, const Scratch &s, float *dbg_cost, float *dbg_agg, cudaStream_t st,
                      bool use_screen = false, int split = 1) {
     const size_t smem = smem_bytes<BH>(g.L, g.min_ds);
     const PadGeom pg = make_pad_geom(g.Hd, g.Wd, g.L, g.min_ds);
     // per-device attribute: set on every launch (cheap) so multi-GPU processes stay correct
-    cudaError_t e = cudaFuncSetAttribute(mbm_wta_fast_kernel<BH, DBG, MODE, STORE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(mbm_wta_fast_kernel<BH, DBG, STORE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     dim3 grid((g.Wd + BW - 1) / BW, (g.Hd + BH - 1) / BH, frames);
     // Whole-volume store (STORE == 1, reference-compat mode): which levels can secondary matching's absolute-index reads
@@ -579,7 +564,7 @@ cudaError_t launch_t(const Geom &g, int frames, const Scratch &s, float *dbg_cos
         store_from = first_level / 2;
     }
     if (STORE == 2) {
-        mbm_wta_fast_kernel<BH, DBG, MODE, STORE, false><<<grid, Cfg<BH>::NT, smem, st>>>(
+        mbm_wta_fast_kernel<BH, DBG, STORE, false><<<grid, Cfg<BH>::NT, smem, st>>>(
             g, pg, s.padl, s.padr, s.wta4, s.edge2, nullptr, nullptr, s.agg_vol, s.gather_mask, s.range_flag, s.range_epoch,
             nullptr, s.bucket_count, 1, nullptr, 0);
         return cudaGetLastError();
@@ -588,9 +573,9 @@ cudaError_t launch_t(const Geom &g, int frames, const Scratch &s, float *dbg_cos
         // level split: every tile's flagged level pairs are spread over `split` blocks writing part slots, then merged
         if (STORE != 0 || DBG || !s.wta4_parts || !s.edge2_parts || !s.part_range) return cudaErrorNotSupported;
         grid.z = frames * split;
-        e = cudaFuncSetAttribute(mbm_wta_fast_kernel<BH, false, MODE, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        e = cudaFuncSetAttribute(mbm_wta_fast_kernel<BH, false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        mbm_wta_fast_kernel<BH, false, MODE, 0, true><<<grid, Cfg<BH>::NT, smem, st>>>(
+        mbm_wta_fast_kernel<BH, false, 0, true><<<grid, Cfg<BH>::NT, smem, st>>>(
             g, pg, s.padl, s.padr, s.wta4_parts, s.edge2_parts, nullptr, nullptr, nullptr, use_screen ? s.pass_mask : nullptr,
             s.range_flag, s.range_epoch, use_screen ? s.tile_order : nullptr, s.bucket_count, split, s.part_range, 0);
         e = cudaGetLastError();
@@ -600,22 +585,10 @@ cudaError_t launch_t(const Geom &g, int frames, const Scratch &s, float *dbg_cos
                                                                       g.Hd, g.Wd, frames, split, pg.tiles_x, pg.tiles_y);
         return cudaGetLastError();
     }
-    mbm_wta_fast_kernel<BH, DBG, MODE, STORE, false><<<grid, Cfg<BH>::NT, smem, st>>>(
+    mbm_wta_fast_kernel<BH, DBG, STORE, false><<<grid, Cfg<BH>::NT, smem, st>>>(
         g, pg, s.padl, s.padr, s.wta4, s.edge2, dbg_cost, dbg_agg, s.agg_vol, use_screen ? s.pass_mask : nullptr,
         s.range_flag, s.range_epoch, use_screen ? s.tile_order : nullptr, s.bucket_count, 1, nullptr, store_from);
     return cudaGetLastError();
-}
-
-int fast_mode() {
-    static int mode = -1;
-    if (mode < 0) {
-        // tuning knob.  bits 0-1: V loop 0 rolled (unroll 2), 1 fully unrolled, 2 manual software pipeline;
-        // (bit 2, C loop fully unrolled, spills registers and was dropped after measurement.)
-        const char *e = getenv("SD_FAST_MODE");
-        mode = e ? atoi(e) : 2;
-        if (mode < 0 || mode > 2) mode = 2;
-    }
-    return mode;
 }
 
 }  // namespace
@@ -631,16 +604,12 @@ cudaError_t launch_mbm_wta_fast(const Geom &g, int frames, const Scratch &s, flo
     if (!mbm_wta_fast_supported(g) || !s.padl || !s.padr) return cudaErrorNotSupported;
     if (gather) {
         if (!s.agg_vol || !s.gather_mask) return cudaErrorNotSupported;
-        return launch_t<32, false, 2, 2>(g, frames, s, nullptr, nullptr, st);
+        return launch_t<32, false, 2>(g, frames, s, nullptr, nullptr, st);
     }
     // the debug / whole-volume modes need every level: no screen there
-    if (dbg_cost || dbg_agg) return launch_t<32, true, 0, 1>(g, frames, s, dbg_cost, dbg_agg, st);
-    if (s.agg_vol) return launch_t<32, false, 2, 1>(g, frames, s, nullptr, nullptr, st);
-    switch (fast_mode()) {
-        case 1: return launch_t<32, false, 1, 0>(g, frames, s, nullptr, nullptr, st, use_screen, split);
-        case 2: return launch_t<32, false, 2, 0>(g, frames, s, nullptr, nullptr, st, use_screen, split);
-        default: return launch_t<32, false, 0, 0>(g, frames, s, nullptr, nullptr, st, use_screen, split);
-    }
+    if (dbg_cost || dbg_agg) return launch_t<32, true, 1>(g, frames, s, dbg_cost, dbg_agg, st);
+    if (s.agg_vol) return launch_t<32, false, 1>(g, frames, s, nullptr, nullptr, st);
+    return launch_t<32, false, 0>(g, frames, s, nullptr, nullptr, st, use_screen, split);
 }
 
 }  // namespace sd

@@ -35,11 +35,9 @@ __device__ __forceinline__ float quad_peak(float x1, float y1, float x2, float y
 }
 
 // NC = number of candidates kept in registers (2K+1); NC == 0: runtime K, neighbours recomputed.
-#ifndef SD_SEC_MIN_BLOCKS
-#define SD_SEC_MIN_BLOCKS 4
-#endif
+// 4 blocks per SM: other occupancy bounds were measured and gave no gain.
 template <int KT>
-__global__ void __launch_bounds__(128, SD_SEC_MIN_BLOCKS) secondary_kernel(Geom g, const float *__restrict__ gray,
+__global__ void __launch_bounds__(128, 4) secondary_kernel(Geom g, const float *__restrict__ gray,
                                                         const float4 *__restrict__ wta4,
                                                         const float2 *__restrict__ edge2, const float *__restrict__ agg_vol,
                                                         const unsigned *__restrict__ gather_mask, PadGeom pg,
