@@ -108,9 +108,20 @@ int sd_set_band(sd_handle *h, int pooled_row_offset, int global_height, const fl
  *   sd_band_p2p_init     the handle must have been created with height = band rows + 2 * halo_rows.  band_row0[world+1]:
  *                        first full-resolution row of every rank's band, band_row0[world] = global height.  Allocates the
  *                        exported buffers and writes this rank's 64-byte CUDA IPC handle to ipc_handle_out.
+ *                        The left-right check and its background fill (sd_set_lr_check / sd_set_lr_fill) must be set
+ *                        before this call and are then fixed for the handle (every rank runs the same exchange steps on
+ *                        every frame): all ranks must use the same settings.  With the check the exported buffer also
+ *                        holds the mirrored frame's left gray band; with the fill, two fill-bounds areas of
+ *                        256 + 8 * W bytes (rounded up to 256) and a third exchange step per frame (DESIGN.md §8).
+ *                        Without the check its size and layout are those of the unchecked mode.  Rectification is
+ *                        refused (SD_ERR_UNSUPPORTED): the remap reads raw rows outside the halo, as far as the maps move
+ *                        rows.
  *   sd_band_p2p_connect  ipc_handles: the world x 64 bytes of all ranks (exchanged by the caller, e.g. an all-gather).
  *   sd_band_p2p_compute  left_band / right_band: [3, band rows, W] of `dtype` (device); out: [band rows + 2 * halo_rows, W]
  *                        floats, rows halo_rows .. halo_rows + band rows - 1 are this rank's part of the disparity map.
+ *                        With the check a call runs one pair (a 2-frame launch); those rows equal sd_compute with the
+ *                        same settings on the whole frame bit for bit, and SD_STAGE_RIGHT (frame 0) returns the right
+ *                        view's map of the window, likewise exact on the band rows.
  * Every rank must call sd_band_p2p_compute the same number of times: a wait that sees no peer for ~10 s gives up (the
  * CUDA context stays usable) and the next sd_band_p2p_compute returns SD_ERR_CUDA with a "timed out" message.
  * sd_destroy on such a handle is COLLECTIVE in effect: peers may still store into / read from the exported buffer, so
@@ -191,8 +202,9 @@ int sd_frames_per_launch(sd_handle *h);
  * Kernels A..C run once per frame and view in shared launches, so a chunk holds frames_per_launch / 2 pairs and a
  * call costs about twice the device time; the fill writes both maps and checks in its epilogue.  Allocates the right
  * maps of one chunk (frames_per_launch / 2 * H * W floats, readable as SD_STAGE_RIGHT); on = 0 frees them and
- * restores the unchecked path exactly.  SD_ERR_SHAPE for a handle created with frames_per_launch = 1;
- * SD_ERR_UNSUPPORTED together with the row-band modes (sd_set_band, sd_band_p2p_init, sd_compute_range). */
+ * restores the unchecked path exactly.  SD_ERR_SHAPE for a handle created with frames_per_launch = 1.
+ * Row bands: supported over peer memory when set BEFORE sd_band_p2p_init (any call on or off after it is
+ * SD_ERR_UNSUPPORTED); the NCCL transport (sd_set_band, sd_compute_range) refuses it, in either order. */
 int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_disparity);
 
 /* Background fill of the pixels the left-right check rejects (KITTI devkit's interpolateBackground), off by default.
@@ -203,8 +215,9 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
  * otherwise stay invalid_disparity (all of them in a frame without a kept pixel).  Every output value is thus a kept
  * left value or invalid_disparity.  With on != 0 the second fill launch of a chunk writes the unchecked left maps and
  * two more launches check and fill them in place.  Allocates frames_per_launch / 2 * H bytes of row flags, freed with
- * the check.  SD_ERR_UNSUPPORTED while the check is off; sd_set_lr_check(h, 0, ...) also switches the fill off, and
- * sd_set_lr_check(h, 1, ...) with the check already on keeps the fill setting. */
+ * the check.  SD_ERR_UNSUPPORTED while the check is off and after sd_band_p2p_init (set it before, like the check);
+ * sd_set_lr_check(h, 0, ...) also switches the fill off, and sd_set_lr_check(h, 1, ...) with the check already on keeps
+ * the fill setting. */
 int sd_set_lr_fill(sd_handle *h, int on);
 
 /* The left-right check plus the background fill (sd_set_lr_fill) without a handle: left_map = n unchecked [H][W] maps,

@@ -21,7 +21,13 @@ Two modes (SURVEY.md section 8-e):
   stores the halo rows straight into the neighbours' HBM while it copies the band into its own window, publishes its
   left gray band for the other ranks' fill kernels to read in place, and synchronises with system-scope flags
   (stereo_depth_b200/csrc/band_p2p.cu).  torch.distributed is then only used once, to exchange the CUDA IPC handles.
+
+  Over peer memory the left-right check (and its background fill) runs on the bands too, bit-identical to a
+  single-GPU `StereoMatching.set_left_right_check` on the whole frame: the mirrored pair is read from the same raw
+  window, the mirrored frame's left gray band is published next to the forward one, and with the fill a third exchange
+  step shares every band's first / last row that kept a pixel (DESIGN.md section 8).
 """
+import math
 from dataclasses import dataclass
 
 import torch
@@ -138,13 +144,30 @@ class BandedStereoMatching:
         sm = BandedStereoMatching(cuda_depth.StereoMatchingConfiguration(height=2160, width=3840, ...))
         out_band = sm.compute(left_band, right_band)     # [3, band_rows, W] each -> [band_rows, W]
         full = sm.gather(out_band)                       # optional: [H, W] on every rank
+
+    left_right_check (a tolerance in pixels, peer-memory transport only) runs the left-right check of
+    `StereoMatching.set_left_right_check` on the bands, with `invalid_disparity` and `background_fill` as there; the
+    band outputs are bit-identical to it on the whole frame.  It is fixed for the object's lifetime (every rank must run
+    the same exchange steps on every frame).
     """
 
-    def __init__(self, configuration, group=None, p2p=False, variant=None):
+    def __init__(self, configuration, group=None, p2p=False, variant=None, left_right_check=None, invalid_disparity=-1.0,
+                 background_fill=False):
         from . import _native as N
         self._N = N
         self.group = group
         self.p2p = bool(p2p)
+        if left_right_check is not None:
+            left_right_check = float(left_right_check)
+            if not math.isfinite(left_right_check) or left_right_check < 0:
+                raise ValueError(f"tolerance must be finite and >= 0, got {left_right_check}")
+            if not self.p2p:
+                raise RuntimeError("the left-right check on row bands needs the peer-memory transport (p2p=True); the "
+                                   "NCCL transport does not support it")
+        elif background_fill:
+            raise RuntimeError("background_fill needs left_right_check (a tolerance in pixels)")
+        self.left_right_check = left_right_check
+        self.background_fill = bool(background_fill) if left_right_check is not None else False
         self._p2p_dtype = None
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -156,9 +179,14 @@ class BandedStereoMatching:
         local = N.SdConfig(*[getattr(g, f) for f in N.CONFIG_FIELDS])
         local.height = self.plan.local_rows
         self.device = torch.cuda.current_device()
-        self.handle = N.Handle(local, self.device, 1)
+        # (with the check a launch carries the frame and its mirrored pair; set before band_p2p_init, which sizes the
+        #  exported buffer for it)
+        self.handle = N.Handle(local, self.device, 1 if left_right_check is None else 2)
         if variant is not None:   # e.g. "fast" pins the screened two-phase kernel (auto decides per launch size)
             self.handle.set_variant({"auto": 0, "generic": 1, "fast": 2, "ws": 3}.get(variant, variant))
+        if left_right_check is not None:
+            self.handle.set_lr_check(True, left_right_check, float(invalid_disparity))
+            self.handle.set_lr_fill(self.background_fill)
         self.H, self.W = g.height, g.width
         self._out = torch.empty((self.plan.local_rows, self.W), dtype=torch.float32, device="cuda")
         self._gray = torch.empty((self.plan.local_rows, self.W), dtype=torch.float32, device="cuda")
@@ -216,6 +244,16 @@ class BandedStereoMatching:
         stream = torch.cuda.current_stream().cuda_stream
         self.handle.band_p2p_compute(left_band.data_ptr(), right_band.data_ptr(), self._out.data_ptr(), stream)
         return self._out[p.halo_rows:p.halo_rows + p.band_rows]
+
+    def right_map(self):
+        """The right view's disparity map (right-image columns) on this rank's band rows, of the last compute() call;
+        needs left_right_check."""
+        if self.left_right_check is None:
+            raise RuntimeError("the right view's map exists only with left_right_check")
+        p = self.plan
+        dst = torch.empty((p.local_rows, self.W), dtype=torch.float32, device="cuda")
+        self.handle.get_stage("right", 0, dst.data_ptr(), torch.cuda.current_stream().cuda_stream)
+        return dst[p.halo_rows:p.halo_rows + p.band_rows]
 
     def gather(self, out_band):
         return gather_rows(out_band, self.rows_per_rank, self.group)

@@ -130,12 +130,17 @@ struct sd_handle {
     Scratch s = {};
     float *dbg_cost = nullptr, *dbg_agg = nullptr;
     GrayView gv = {};      // band mode: where the left gray of the global image lives, else all zero
-    // peer-memory row bands (sd_band_p2p_*): one exported allocation per rank = [window L | window R | gray 0 | gray 1 | flags]
+    GrayView gv_mir = {};  // peer-memory band mode with the left-right check: the same for the mirrored frames' left gray
+    // peer-memory row bands (sd_band_p2p_*): one exported allocation per rank =
+    //   [window L | window R | gray 0 | gray 1 | flags | fill 0 | fill 1]
+    // gray p holds one plane per frame of a call (two with the left-right check: forward, mirrored); the fill areas
+    // (FillAreas in common.cuh) exist only with the background fill
     struct P2P : NoCopy {
         bool on = false, connected = false;
         int world = 0, rank = 0, dtype = 0, halo_rows = 0;
         int row0[9] = {};            // full-resolution first row of every rank's band (+ total height)
         size_t win_bytes = 0, gray_bytes = 0;  // per window / per published gray buffer (sized for the tallest band)
+        size_t gray_plane_bytes = 0, fill_bytes = 0;  // per plane of a gray buffer / per fill area (0 without the fill)
         char *base = nullptr;        // my allocation
         char *peer[8] = {};          // every rank's allocation (peer[rank] == base)
         unsigned epoch = 0;
@@ -447,11 +452,16 @@ int run_chunk(sd_handle *h, const void *left, const void *right, int dtype, int 
         Scratch mirrored = h->s;   // the fill of frames pairs..2*pairs-1
         mirrored.gray += (size_t)pairs * 2 * n;
         mirrored.refined += (size_t)pairs * nd;
-        SD_CUDA(h, launch_fill(h->g, pairs, mirrored, h->gv, h->rmap, st));
+        // (peer-memory row bands: the mirrored frame's colour rows come from the ranks' published mirrored gray bands)
+        SD_CUDA(h, launch_fill(h->g, pairs, mirrored, h->gv.n > 0 ? h->gv_mir : h->gv, h->rmap, st));
         if (h->lr_fill) {   // unchecked left maps, then the check and the background fill in place
             SD_CUDA(h, launch_fill(h->g, pairs, h->s, h->gv, out, st));
-            SD_CUDA(h, launch_lr_background_fill(out, h->rmap, true, pairs, h->g.H, h->g.W, h->lr_tol, h->lr_invalid, out,
-                                                 h->lr_rows, st));
+            if (h->gv.n == 0)
+                SD_CUDA(h, launch_lr_background_fill(out, h->rmap, true, pairs, h->g.H, h->g.W, h->lr_tol, h->lr_invalid,
+                                                     out, h->lr_rows, st));
+            else   // peer-memory row bands: the column pass follows the fill-bounds exchange (sd_band_p2p_compute)
+                SD_CUDA(h, launch_lr_fill_rows(out, h->rmap, pairs, h->g.H, h->g.W, h->lr_tol, h->lr_invalid, out,
+                                               h->lr_rows, st));
         } else {
             SD_CUDA(h, launch_fill_lr(h->g, pairs, h->s, h->gv, out, LrCheck{h->rmap, h->lr_tol, h->lr_invalid}, st));
         }
@@ -743,12 +753,16 @@ int sd_set_band(sd_handle *h, int pooled_row_offset, int global_height, const fl
 // ---- row bands over peer memory ------------------------------------------------------------------------------------
 namespace {
 constexpr size_t kP2PFlagBytes = 4096;
-enum { kFlagFromPrev = 0, kFlagFromNext = 1, kFlagGray = 8, kCtrScatter = 32, kCtrPublish = 33 };
+enum { kFlagFromPrev = 0, kFlagFromNext = 1, kFlagGray = 8, kFlagFill = 16, kCtrScatter = 32, kCtrPublish = 33, kCtrFill = 34 };
 inline char *p2p_window(const sd_handle *h, int q, int view) { return h->p2p.peer[q] + (size_t)view * h->p2p.win_bytes; }
-inline float *p2p_gray(const sd_handle *h, int q, int parity) {
-    return (float *)(h->p2p.peer[q] + 2 * h->p2p.win_bytes + (size_t)parity * h->p2p.gray_bytes);
+inline float *p2p_gray(const sd_handle *h, int q, int parity, int plane = 0) {
+    return (float *)(h->p2p.peer[q] + 2 * h->p2p.win_bytes + (size_t)parity * h->p2p.gray_bytes +
+                     (size_t)plane * h->p2p.gray_plane_bytes);
 }
 inline unsigned *p2p_flags(const sd_handle *h, int q) { return (unsigned *)(h->p2p.peer[q] + 2 * h->p2p.win_bytes + 2 * h->p2p.gray_bytes); }
+inline float *p2p_fill(const sd_handle *h, int q, int parity) {
+    return (float *)((char *)p2p_flags(h, q) + kP2PFlagBytes + (size_t)parity * h->p2p.fill_bytes);
+}
 }  // namespace
 
 int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0, int halo_rows, int dtype, void *ipc_handle_out) {
@@ -756,7 +770,6 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     if (world < 1 || world > 8 || rank < 0 || rank >= world) return fail(h, SD_ERR_BAD_ARG, "peer-memory band mode supports 1..8 ranks");
     if (dtype != SD_U8 && dtype != SD_F32) return fail(h, SD_ERR_SHAPE, "dtype must be SD_U8 or SD_F32");
     if (h->p2p.on) return fail(h, SD_ERR_BAD_ARG, "sd_band_p2p_init was already called on this handle");
-    if (h->lr) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check (sd_set_lr_check(h, 0, ...) first)");
     if (h->rect_maps) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support rectification (sd_set_rectification(h, NULL, ...) first)");
     const Geom &g = h->g;
     const int esize = dtype == SD_U8 ? 1 : 4, K = g.K;
@@ -783,8 +796,11 @@ int sd_band_p2p_init(sd_handle *h, int world, int rank, const int32_t *band_row0
     p.halo_rows = halo_rows;
     for (int q = 0; q <= world; q++) p.row0[q] = band_row0[q];
     p.win_bytes = (((size_t)3 * (tallest + 2 * halo_rows) * g.W * esize) + 255) & ~(size_t)255;
-    p.gray_bytes = (((size_t)tallest * g.W * sizeof(float)) + 255) & ~(size_t)255;
-    const size_t total = 2 * p.win_bytes + 2 * p.gray_bytes + kP2PFlagBytes;
+    // (the left-right check adds the mirrored frame's gray plane, its background fill the two fill areas)
+    p.gray_plane_bytes = (((size_t)tallest * g.W * sizeof(float)) + 255) & ~(size_t)255;
+    p.gray_bytes = (h->lr ? 2 : 1) * p.gray_plane_bytes;
+    p.fill_bytes = h->lr_fill ? fill_area_bytes(g.W) : 0;
+    const size_t total = 2 * p.win_bytes + 2 * p.gray_bytes + kP2PFlagBytes + 2 * p.fill_bytes;
     SD_CUDA(h, cudaMalloc((void **)&p.base, total));
     cudaIpcMemHandle_t ipc;
     cudaError_t e = cudaMemset(p.base, 0, total);
@@ -850,7 +866,8 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
                                    myflags + kCtrScatter, p2p_flags(h, prev) + kFlagFromNext, p2p_flags(h, next) + kFlagFromPrev,
                                    epoch, st));
     SD_CUDA(h, launch_wait_flags(myflags, kFlagFromPrev, 2, epoch, p.timeout.dev, st));
-    // gray + pool on the local window [top halo | band | bottom halo]
+    // gray + pool on the local window [top halo | band | bottom halo] (with the left-right check: frame 0 and the mirrored
+    // frame 1 of the pair, read from the same window -- mirroring reverses columns only)
     // (h->g is the handle's own geometry and is rewritten for the two halves of every frame: a handle is not
     //  thread-safe -- include/stereo_b200.h -- and the kernels receive Geom by value, so launches already in flight keep
     //  the values they were given)
@@ -860,12 +877,18 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
     memset(&h->gv, 0, sizeof(h->gv));
     rc = run_chunk(h, p2p_window(h, r, 0), p2p_window(h, r, 1), p.dtype, 1, out, st, 0, 0);
     if (rc != SD_OK) return rc;
-    // exchange step 2: publish my left gray band, tell every rank (myself included)
+    // exchange step 2: publish my left gray band (with the check also the mirrored frame's), tell every rank (myself
+    // included)
     const int parity = (int)(epoch & 1u);
     unsigned *peer_flags[8];
     for (int q = 0; q < n; q++) peer_flags[q] = p2p_flags(h, q) + kFlagGray + r;
-    SD_CUDA(h, launch_publish_gray(h->s.gray + (size_t)halo * W, p2p_gray(h, r, parity), (size_t)band_rows * W,
-                                   myflags + kCtrPublish, peer_flags, n, epoch, st));
+    if (h->lr)
+        SD_CUDA(h, launch_publish_gray(h->s.gray + (size_t)halo * W, p2p_gray(h, r, parity), (size_t)band_rows * W,
+                                       myflags + kCtrPublish, peer_flags, n, epoch, st, 2, (size_t)2 * g.H * W,
+                                       p.gray_plane_bytes / sizeof(float)));
+    else
+        SD_CUDA(h, launch_publish_gray(h->s.gray + (size_t)halo * W, p2p_gray(h, r, parity), (size_t)band_rows * W,
+                                       myflags + kCtrPublish, peer_flags, n, epoch, st));
     SD_CUDA(h, launch_wait_flags(myflags, kFlagGray, n, epoch, p.timeout.dev, st));
     // matching + secondary + fill on the window; the fill reads its colour row from whichever rank owns it
     h->g.band_x_off = (p.row0[r] - halo) / g.K;
@@ -877,8 +900,23 @@ int sd_band_p2p_compute(sd_handle *h, const void *left_band, const void *right_b
         h->gv.row0[q] = p.row0[q];
     }
     h->gv.row0[n] = p.row0[n];
+    h->gv_mir = h->gv;
+    for (int q = 0; q < n; q++) h->gv_mir.band[q] = p2p_gray(h, q, parity, 1);
     rc = run_chunk(h, nullptr, nullptr, p.dtype, 1, out, st, 1, 3);
     if (rc != SD_OK) return rc;
+    if (h->lr_fill) {
+        // exchange step 3: the column pass of the background fill needs the frame's first / last row that kept a pixel,
+        // which can lie on any rank.  Publish my band's bounds and rows, wait for every rank's, fill my band rows.
+        unsigned *fill_flags[8];
+        for (int q = 0; q < n; q++) fill_flags[q] = p2p_flags(h, q) + kFlagFill + r;
+        SD_CUDA(h, launch_publish_fill_bounds(h->lr_rows + halo, out + (size_t)halo * W, band_rows, p.row0[r], W,
+                                              p2p_fill(h, r, parity), myflags + kCtrFill, fill_flags, n, epoch, st));
+        SD_CUDA(h, launch_wait_flags(myflags, kFlagFill, n, epoch, p.timeout.dev, st));
+        FillAreas areas = {};
+        areas.n = n;
+        for (int q = 0; q < n; q++) areas.area[q] = p2p_fill(h, q, parity);
+        SD_CUDA(h, launch_lr_fill_cols_band(out, h->lr_rows, halo, band_rows, p.row0[r], W, areas, st));
+    }
     return mark_last_use(h, st);
 }
 
@@ -1059,6 +1097,10 @@ int sd_frames_per_launch(sd_handle *h) { return h ? h->chunk : 0; }
 
 int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_disparity) {
     if (!h) return SD_ERR_BAD_ARG;
+    // (every rank must run the same exchange steps on every frame, and the exported buffer is sized for the mode)
+    if (h->p2p.on)
+        return fail(h, SD_ERR_UNSUPPORTED, "the left-right check of a peer-memory band handle is fixed at sd_band_p2p_init: "
+                                           "set it before sd_band_p2p_init");
     if (!on) {
         if (h->rmap) {
             DeviceGuard dg(h->device);
@@ -1074,7 +1116,7 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
     if (h->chunk < 2)
         return fail(h, SD_ERR_SHAPE, "the left-right check runs each frame together with its mirrored pair: create the handle "
                                      "with frames_per_launch >= 2");
-    if (h->gv.flat || h->p2p.on) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check");
+    if (h->gv.flat) return fail(h, SD_ERR_UNSUPPORTED, "row-band mode does not support the left-right check");
     if (!h->rmap) {
         DeviceGuard dg(h->device);
         if (!dg.ok) return fail(h, SD_ERR_CUDA, "cudaSetDevice failed");
@@ -1088,6 +1130,9 @@ int sd_set_lr_check(sd_handle *h, int on, float tolerance, float invalid_dispari
 
 int sd_set_lr_fill(sd_handle *h, int on) {
     if (!h) return SD_ERR_BAD_ARG;
+    if (h->p2p.on)
+        return fail(h, SD_ERR_UNSUPPORTED, "the background fill of a peer-memory band handle is fixed at sd_band_p2p_init: "
+                                           "set it before sd_band_p2p_init");
     if (!h->lr) return fail(h, SD_ERR_UNSUPPORTED, "the background fill needs the left-right check (sd_set_lr_check(h, 1, ...) first)");
     if (on && !h->lr_rows) {
         DeviceGuard dg(h->device);

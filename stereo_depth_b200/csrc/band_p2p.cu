@@ -6,10 +6,14 @@
 //                         circular, device_functions.cuh:13-14).  The last block to finish releases the two flags.
 //   publish_gray_kernel   my left gray band -> my published buffer (double buffered by frame parity); the last block
 //                         releases one flag at every peer.  The fill kernel then reads the one row it needs,
-//                         GL[(K+1)x] (upscale_disparity_vertical_fill.cu:31), from whichever rank owns it.
+//                         GL[(K+1)x] (upscale_disparity_vertical_fill.cu:31), from whichever rank owns it.  With the
+//                         left-right check it publishes the mirrored frame's left gray band too (second plane).
+//   publish_fill_bounds_kernel  (background fill of the check only) my band's first / last row that kept a pixel and
+//                         copies of those two rows -> my fill area (double buffered by frame parity); the last block
+//                         releases one flag at every peer.  The column pass then applies the frame's global rule.
 //   wait_flags_kernel     one warp spins (ld.acquire.sys) until the flags it is given reach the frame's epoch.
 //
-// Ordering argument (why single windows and two gray buffers suffice) is in DESIGN.md section 8.
+// Ordering argument (why single windows, two gray buffers and two fill areas suffice) is in DESIGN.md section 8.
 #include "common.cuh"
 
 namespace sd {
@@ -70,10 +74,52 @@ struct PeerFlags {
     int n;
 };
 
+// (planes > 1 with the left-right check: the forward and the mirrored frame's left gray band, strides in float4)
 __global__ void __launch_bounds__(256) publish_gray_kernel(const float4 *__restrict__ src, float4 *__restrict__ dst, size_t n4,
-                                                           unsigned *counter, PeerFlags peers, unsigned epoch) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) dst[i] = __ldg(src + i);
+                                                           unsigned *counter, PeerFlags peers, unsigned epoch, int planes,
+                                                           size_t src_plane4, size_t dst_plane4) {
+    for (int pl = 0; pl < planes; pl++)
+        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x)
+            dst[pl * dst_plane4 + i] = __ldg(src + pl * src_plane4 + i);
     if (last_block_done(counter, gridDim.x) && threadIdx.x < peers.n) st_release_sys(peers.p[threadIdx.x], epoch);
+}
+
+// Fill-bounds exchange (background fill of the left-right check, DESIGN.md §13): block (x, y) copies segment x of the
+// band's first (y = 0) or last (y = 1) row that kept a pixel; every block finds the two rows itself from the band's row
+// flags (a few hundred bytes).  Block (0, 0) writes their global rows; the last block releases one flag at every peer.
+__global__ void __launch_bounds__(256) publish_fill_bounds_kernel(const unsigned char *__restrict__ row_kept,
+                                                                  const float *__restrict__ rows, int band_rows, int glob_row0,
+                                                                  int W, float *area, unsigned *counter, PeerFlags peers,
+                                                                  unsigned epoch) {
+    __shared__ int sh_first[8], sh_last[8];
+    int first = 0x7fffffff, last = -1;
+    for (int i = threadIdx.x; i < band_rows; i += 256)
+        if (row_kept[i]) {
+            first = min(first, i);
+            last = max(last, i);
+        }
+    first = __reduce_min_sync(0xffffffffu, first);
+    last = __reduce_max_sync(0xffffffffu, last);
+    if ((threadIdx.x & 31) == 0) {
+        sh_first[threadIdx.x >> 5] = first;
+        sh_last[threadIdx.x >> 5] = last;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int w = 0; w < 8; w++) {
+        first = min(first, sh_first[w]);
+        last = max(last, sh_last[w]);
+    }
+    if (last >= 0) {
+        const float *s = rows + (size_t)(blockIdx.y ? last : first) * W;
+        float *d = area + kFillAreaHeaderFloats + (size_t)blockIdx.y * W;
+        for (int c = blockIdx.x * 256 + threadIdx.x; c < W; c += gridDim.x * 256) d[c] = s[c];
+    }
+    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
+        reinterpret_cast<int *>(area)[0] = last >= 0 ? glob_row0 + first : -1;
+        reinterpret_cast<int *>(area)[1] = last >= 0 ? glob_row0 + last : -1;
+    }
+    if (last_block_done(counter, gridDim.x * gridDim.y) && threadIdx.x < peers.n) st_release_sys(peers.p[threadIdx.x], epoch);
 }
 
 // A missing peer must neither hang the GPU nor poison the CUDA context: after ~10 s the waiting lane posts
@@ -111,16 +157,34 @@ cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l
     return cudaGetLastError();
 }
 
-cudaError_t launch_publish_gray(const float *src, float *dst, size_t n_floats, unsigned *counter, unsigned *const *peer_flags,
-                                int n_peers, unsigned epoch, cudaStream_t st) {
+namespace {
+PeerFlags peer_flags_of(unsigned *const *peer_flags, int n_peers) {
     PeerFlags pf;
     pf.n = n_peers;
     for (int i = 0; i < 8; i++) pf.p[i] = i < n_peers ? peer_flags[i] : nullptr;
+    return pf;
+}
+}  // namespace
+
+cudaError_t launch_publish_gray(const float *src, float *dst, size_t n_floats, unsigned *counter, unsigned *const *peer_flags,
+                                int n_peers, unsigned epoch, cudaStream_t st, int planes, size_t src_plane, size_t dst_plane) {
+    const PeerFlags pf = peer_flags_of(peer_flags, n_peers);
     const size_t n4 = n_floats / 4;
     int blocks = (int)((n4 + 255) / 256);
     if (blocks > 592) blocks = 592;
     if (blocks < 1) blocks = 1;
-    publish_gray_kernel<<<blocks, 256, 0, st>>>((const float4 *)src, (float4 *)dst, n4, counter, pf, epoch);
+    publish_gray_kernel<<<blocks, 256, 0, st>>>((const float4 *)src, (float4 *)dst, n4, counter, pf, epoch, planes,
+                                                src_plane / 4, dst_plane / 4);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_publish_fill_bounds(const unsigned char *row_kept, const float *rows, int band_rows, int glob_row0, int W,
+                                       float *area, unsigned *counter, unsigned *const *peer_flags, int n_peers,
+                                       unsigned epoch, cudaStream_t st) {
+    const PeerFlags pf = peer_flags_of(peer_flags, n_peers);
+    int seg = (W + 1023) / 1024;   // (about 4 columns per thread)
+    if (seg > 16) seg = 16;
+    publish_fill_bounds_kernel<<<dim3(seg, 2), 256, 0, st>>>(row_kept, rows, band_rows, glob_row0, W, area, counter, pf, epoch);
     return cudaGetLastError();
 }
 

@@ -166,6 +166,25 @@ cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const Gr
 cudaError_t launch_lr_background_fill(const float *left, const float *right, bool right_mirrored, int frames, int H, int W,
                                       float tolerance, float invalid, float *out, unsigned char *row_kept,
                                       cudaStream_t st);
+// The row pass of launch_lr_background_fill alone (right map mirrored): the peer-memory row-band mode runs its column
+// pass only after the fill-bounds exchange (launch_lr_fill_cols_band).
+cudaError_t launch_lr_fill_rows(const float *left, const float *right_mirrored, int frames, int H, int W, float tolerance,
+                                float invalid, float *out, unsigned char *row_kept, cudaStream_t st);
+// Fill-bounds area of one rank and frame parity (peer-memory row bands with the background fill, DESIGN.md §8 / §13):
+//   int [0] / [1]: first / last GLOBAL row of the rank's band that kept a pixel (-1: none), padded to 256 bytes;
+//   then floats [W]: that first row after the row pass, and [W]: that last row.
+constexpr int kFillAreaHeaderFloats = 64;
+inline size_t fill_area_bytes(int W) { return ((size_t)kFillAreaHeaderFloats * 4 + 8 * (size_t)W + 255) & ~(size_t)255; }
+struct FillAreas {
+    const float *area[8];   // every rank's area of this frame's parity, in rank (= row) order
+    int n;
+};
+// Column pass of the background fill on the band rows [row_first, row_first + band_rows) of one local window `out`
+// (row_kept: the row pass's flags of the same window; glob_row0: global row of local row row_first): a row without a
+// kept pixel copies the frame's first non-empty row when it lies above it, the last one when below it, read from the
+// published copy of the rank that owns it.  Writes nothing outside the band.
+cudaError_t launch_lr_fill_cols_band(float *out, const unsigned char *row_kept, int row_first, int band_rows, int glob_row0,
+                                     int W, const FillAreas &areas, cudaStream_t st);
 // Rectification remap (rectify.cu, DESIGN.md §14), exactly cv2.remap with CV_32FC1 maps, INTER_LINEAR and a constant 0
 // border: dst[p][r][c] = src[p] sampled at (map_x[r][c], map_y[r][c]) for `planes` [H][W] planes per view, uint8 or
 // float32 by `dtype`; grid.y runs over the n_views (1 or 2) views.  H, W < 32768; dst must not overlap src.
@@ -191,8 +210,16 @@ cudaError_t launch_band_scatter(const void *left, const void *right, void *own_l
                                 void *next_l, void *next_r, int row_bytes, int band_rows, int halo, int own_rows, int prev_rows,
                                 int next_rows, unsigned *counter, unsigned *flag_at_prev, unsigned *flag_at_next, unsigned epoch,
                                 cudaStream_t st);
+// `planes` planes of n_floats each: plane i from src + i * src_plane to dst + i * dst_plane (floats)
 cudaError_t launch_publish_gray(const float *src, float *dst, size_t n_floats, unsigned *counter, unsigned *const *peer_flags,
-                                int n_peers, unsigned epoch, cudaStream_t st);
+                                int n_peers, unsigned epoch, cudaStream_t st, int planes = 1, size_t src_plane = 0,
+                                size_t dst_plane = 0);
+// Fill-bounds exchange: finds the first / last kept row among the band's `band_rows` row flags, copies those two filled
+// rows of `rows` ([band_rows][W]) and their global rows (glob_row0 + index) into `area` (my fill area, layout above),
+// then releases one flag at every peer.
+cudaError_t launch_publish_fill_bounds(const unsigned char *row_kept, const float *rows, int band_rows, int glob_row0, int W,
+                                       float *area, unsigned *counter, unsigned *const *peer_flags, int n_peers,
+                                       unsigned epoch, cudaStream_t st);
 cudaError_t launch_wait_flags(const unsigned *flags, int first, int count, unsigned epoch, unsigned long long *timeout_word,
                               cudaStream_t st);
 

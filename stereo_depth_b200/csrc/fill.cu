@@ -377,6 +377,38 @@ __global__ void __launch_bounds__(256) lr_fill_cols_kernel(float *out, const uns
     for (int c = threadIdx.x; c < W; c += 256) o[c] = s[c];
 }
 
+// Column pass of one row band (peer-memory row-band mode, DESIGN.md §8): the same rule with the frame's GLOBAL first /
+// last non-empty row, taken from every rank's published fill bounds in rank order, and the row to copy read from the
+// published copy of the rank that owns it.  One block per band row; blocks of non-empty rows return at once.
+__global__ void __launch_bounds__(256) lr_fill_cols_band_kernel(float *out, const unsigned char *__restrict__ row_kept,
+                                                                int row_first, int glob_row0, int W, const FillAreas areas) {
+    const int r = row_first + blockIdx.x;
+    if (row_kept[r]) return;
+    int first = -1, last = -1;
+    const float *src_first = nullptr, *src_last = nullptr;
+    // compile-time indices only: the areas stay in the kernel's parameter space (no local copy)
+#pragma unroll
+    for (int q = 0; q < 8; q++)
+        if (q < areas.n) {
+            const float *a = areas.area[q];
+            const int f = reinterpret_cast<const int *>(a)[0];
+            if (f >= 0) {
+                if (first < 0) {
+                    first = f;
+                    src_first = a + kFillAreaHeaderFloats;
+                }
+                last = reinterpret_cast<const int *>(a)[1];
+                src_last = a + kFillAreaHeaderFloats + W;
+            }
+        }
+    if (last < 0) return;   // no kept pixel in the frame: all `invalid`
+    const int rg = glob_row0 + (int)blockIdx.x;
+    const float *s = rg < first ? src_first : (rg > last ? src_last : nullptr);
+    if (!s) return;
+    float *o = out + (size_t)r * W;
+    for (int c = threadIdx.x; c < W; c += 256) o[c] = s[c];
+}
+
 template <bool LR>
 cudaError_t fill(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
                  cudaStream_t st) {
@@ -405,6 +437,19 @@ cudaError_t launch_fill(const Geom &g, int frames, const Scratch &s, const GrayV
 cudaError_t launch_fill_lr(const Geom &g, int frames, const Scratch &s, const GrayView &gl_glob, float *out, const LrCheck &lr,
                            cudaStream_t st) {
     return fill<true>(g, frames, s, gl_glob, out, lr, st);
+}
+
+cudaError_t launch_lr_fill_rows(const float *left, const float *right_mirrored, int frames, int H, int W, float tolerance,
+                                float invalid, float *out, unsigned char *row_kept, cudaStream_t st) {
+    lr_fill_rows_kernel<true><<<(unsigned)frames * (unsigned)H, kBgThreads, 0, st>>>(left, right_mirrored, out, row_kept, W,
+                                                                                    tolerance, invalid);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_lr_fill_cols_band(float *out, const unsigned char *row_kept, int row_first, int band_rows, int glob_row0,
+                                     int W, const FillAreas &areas, cudaStream_t st) {
+    lr_fill_cols_band_kernel<<<band_rows, 256, 0, st>>>(out, row_kept, row_first, glob_row0, W, areas);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_lr_background_fill(const float *left, const float *right, bool right_mirrored, int frames, int H, int W,
